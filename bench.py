@@ -5,7 +5,7 @@ Workload = BASELINE config C3: the fused FK + Jacobian + QP + J^T f torque pipel
 states per GPU, FP64 (weak scaling: every rank owns its own 2^20-state slice of the counter-based
 synthetic batch; no collective on the solve path, one tiny NCCL all-reduce of statistics at the end).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  `value` = whole-job QP/s with inputs resident in HBM; `e2e` = the same
@@ -13,6 +13,9 @@ through the C ABI's host-pointer entry (pinned host buffers, H2D + D2H inside th
 `roofline` = algorithmic FP64 FLOP/s of the fused kernel against the FP64 FMA peak measured on the box;
 `cpu_baseline` = the reference's own QuadProg++ (oracle/_ref) or the oracle port on the host cores.
 --impl reference times that CPU path alone.
+--dump-outputs DIR also writes what the timed solve call returned in its last step (grf, tau, netwrench, flags of
+rank 0's slice) as DIR/<name>.npy; the inputs are the same on every run with the same arguments, so two builds can
+be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,6 +53,23 @@ def bench_config(B: int, world: int) -> dict:
 
 
 NCU_RECORD = os.path.join(ROOT, "profiles", "r2_final_ncu.json")   # written by tools/ncu_summary.py from the committed capture
+DUMP_STATES = 1 << 17   # states written by --dump-outputs: 31 FP64 values each, 32.5 MB in all
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """Write the [C, B] device outputs of one solve call as out_dir/<name>.npy in float64 (flags too: every uint32 is
+    exact there).  A batch larger than DUMP_STATES is sampled: the same seeded, sorted state indices for a given batch
+    size on every run."""
+    import torch
+    B = outputs["flags"].shape[-1]
+    idx = np.arange(B) if B <= DUMP_STATES else np.sort(np.random.default_rng(0).choice(B, DUMP_STATES, replace=False))
+    sel = torch.from_numpy(idx).to(outputs["flags"].device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.index_select(-1, sel).cpu().numpy()
+        if name == "flags":
+            a = a.view(np.uint32)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 _JSON_FD = None   # the process's real stdout once emit_only_json_on_stdout() has moved fd 1 to stderr
@@ -247,6 +267,8 @@ def run_sweep(args, rank, local_rank, world, dev, warmup):
     launches0 = solver.launches
     ms_step = timed(solve, args.steps)
     launches = solver.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"grf": grf, "tau": tau, "netwrench": net, "flags": flags})
     ms_gen = timed(generate, max(3, args.steps // 4))
 
     stats_holder = {}
@@ -304,7 +326,14 @@ def main():
     ap.add_argument("--batch", type=int, default=BATCH_PER_GPU, help="states per GPU (default 2^20)")
     ap.add_argument("--config", default="C3")
     ap.add_argument("--cpu-sample", type=int, default=1 << 19)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help=f"write the outputs of the last timed step as DIR/<name>.npy (a fixed sample of {DUMP_STATES} states "
+                         "when the batch is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     warmup = max(3, args.warmup)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -391,6 +420,8 @@ def main():
     ev1.record(stream)
     barrier()
     launches = solver.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"grf": grf, "tau": tau, "netwrench": net, "flags": flags})
     ms_total = ev0.elapsed_time(ev1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:

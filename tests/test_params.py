@@ -1,6 +1,7 @@
 """Parameters under the reference's own names: qlb_params_set_key / qlb_params_from_yaml (host code, runs without
 a GPU) and the adapter classes' loadParameters() (GPU)."""
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -87,18 +88,22 @@ def test_yaml_fills_the_parameter_block(qlb_built):
     assert missing is None and [p.kp_translation[0], p.kd_translation[0], p.kff_translation[0]] == [1.0, 2.0, 3.0]
 
 
+def _yaml(tree: dict, indent: str = "") -> str:
+    return "".join(f"{indent}{k}:\n" + _yaml(v, indent + "  ") if isinstance(v, dict) else f"{indent}{k}: {v!r}\n"
+                   for k, v in tree.items())
+
+
 def test_defaults_are_the_references_file(qlb_built):
-    """Where the reference tree is available (the build container): its own controller_gains.yaml reproduces
-    qlb_default_params exactly."""
-    path = "/root/reference/balance_controller/config/controller_gains.yaml"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    """The values of the reference's controller_gains.yaml (tests/golden/controller_gains.json, written out again in
+    the file's layout) reproduce qlb_default_params exactly."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "controller_gains.json")) as f:
+        text = _yaml(json.load(f)["parameters"])
     p0 = capi.default_params()
     zero = capi.default_params()
     lib = capi.load()
     for i in range(lib.qlb_params_num_keys()):
         lib.qlb_params_set_key(C.byref(zero), lib.qlb_params_key(i), -1.0)
-    p, missing = capi.params_from_yaml(open(path).read(), base=zero)
+    p, missing = capi.params_from_yaml(text, base=zero)
     assert missing is None
     assert bytes(p) == bytes(p0)
 
