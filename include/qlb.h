@@ -397,6 +397,67 @@ int qlb_contact_fsm(qlb_context* ctx, size_t B, const uint8_t* desired_stance_ma
                     const uint8_t* contact_mask, const double* phase, uint8_t* limb_state, uint8_t* stance_mask,
                     void* stream);
 
+/* ---- the controller tick for B robots (RosBalanceController::update / starting) --------------------------------
+ * One qlb_controller_update = one 2.5 ms tick of ros_balance_controller.cpp:198-716 for every robot of the batch:
+ * contact state machine (as qlb_contact_fsm) -> state-mode solve of the stance legs (as qlb_solve_state) -> swing-leg
+ * torques with the velocity-queue acceleration (as qlb_swing_leg_torques_from_queue) -> merge into the robot's joint
+ * efforts -> clamped command.  The state that lives from tick to tick is kept on the device, per robot:
+ *   limb_state[4][B]  qlb_limb_state per leg; QLB_LIMB_INIT after create / reset
+ *   efforts[12][B]    the reference's State joint efforts: unclamped, zero after create / reset, never non-finite.
+ *                     Stance rows take the solve's torques when its status is QLB_STATE_OK or QLB_STATE_NO_STANCE and
+ *                     keep their previous value otherwise (stale efforts, RBC.cpp:418,455-458); swing rows take the
+ *                     swing-leg torques unless one of the leg's three is non-finite, in which case the row is kept
+ *   a ring of the last 11 joint-velocity samples qd: the newest is this tick's sample, the oldest the one 10 ticks
+ *                     earlier, so the swing legs use qdd = (qd_newest - qd_oldest) / (10 period), the reference's
+ *                     Time_derta divisor over a true 10-period span.  Start-up rule: the first tick after create or
+ *                     reset fills all 11 samples of the robot with its qd, so that tick has qdd = 0; a non-finite qd
+ *                     sample makes that robot's swing rows stale until it has left the ring (10 ticks).
+ * A controller and its arrays belong to one context: destroy the controller before the context.  Updates of one
+ * controller must be ordered (one stream, or the caller orders them); every update is ordered after the controller's
+ * last reset, whatever stream that ran on; different controllers of one context may run on different streams at the
+ * same time.  Every update launches the kernels of qlb_solve_state plus two.  After an update that returned an error the
+ * robots' state is unspecified until they are reset. */
+typedef struct qlb_tick_params {
+  double period;           /* control period in s: 0.0025 (400 Hz, balance_controller_manager.cpp:48,70) */
+  double effort_limit;     /* |command| clamp in N m: 300 (RBC.cpp:450-454); the stored efforts are not clamped */
+  qlb_swing_params swing;  /* swing-leg gains and gravity, as qlb_default_swing_params */
+} qlb_tick_params;         /* 96 bytes */
+int qlb_default_tick_params(qlb_tick_params* p);
+
+typedef struct qlb_controller qlb_controller;
+/* Allocates the per-robot state for B robots on ctx's device (limb states INIT, efforts zero, rings marked for refill)
+ * and synchronises.  The swing legs need the limb tables: qlb_set_limb_dynamics before the first update.
+ * QLB_ERR_CUDA when no CUDA device is usable. */
+int qlb_controller_create(qlb_context* ctx, size_t B, const qlb_tick_params* params, qlb_controller** out);
+int qlb_controller_destroy(qlb_controller* c);
+/* RosBalanceController::starting for the robots with reset_mask[i] != 0 (DEVICE [B]; NULL = all): limb states INIT,
+ * efforts zero, ring refilled by the next sample.  Other robots are untouched.  Asynchronous on `stream`. */
+int qlb_controller_reset(qlb_controller* c, const uint8_t* reset_mask, void* stream);
+/* One tick for all B robots, DEVICE pointers, asynchronous on `stream`.
+ *   q[12][B], qd[12][B]           measured joint positions and velocities
+ *   base_pose .. target_twist     as qlb_solve_state
+ *   desired_stance_mask, footstep_mask (NULL = all legs), contact_mask, phase[4][B]   as qlb_contact_fsm
+ *   mu, normals_world             as qlb_solve_state (NULL ok)
+ *   foot_target_position, foot_target_velocity   as qlb_swing_leg_torques (NULL ok: that error term is zero)
+ *   command[12][B]                out: clamp(efforts, +-effort_limit)
+ *   flags[B]                      out: result word of the solve
+ *   grf[12][B]                    out (NULL ok): ground-reaction forces of the solve */
+int qlb_controller_update(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
+                          const double* base_twist, const double* target_pose, const double* target_twist,
+                          const uint8_t* desired_stance_mask, const uint8_t* footstep_mask, const uint8_t* contact_mask,
+                          const double* phase, const double* mu, const double* normals_world,
+                          const double* foot_target_position, const double* foot_target_velocity, double* command,
+                          uint32_t* flags, double* grf, void* stream);
+/* Same, HOST pointers: staged through the context's buffers, synchronises (a batch-of-1 controller tick). */
+int qlb_controller_update_host(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
+                               const double* base_twist, const double* target_pose, const double* target_twist,
+                               const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
+                               const uint8_t* contact_mask, const double* phase, const double* mu,
+                               const double* normals_world, const double* foot_target_position,
+                               const double* foot_target_velocity, double* command, uint32_t* flags, double* grf);
+/* DEVICE copies of the persistent state, asynchronous on `stream`: limb_state[4][B], efforts[12][B] (either NULL ok). */
+int qlb_controller_get_state(const qlb_controller* c, uint8_t* limb_state, double* efforts, void* stream);
+
 /* Friction margins of a solved batch (DEVICE pointers): margin[i] = min over stance legs and the four friction rows of
  * slack / (mu n.f) - 1 = unloaded tangentially, 0 = a friction row is active; min_normal[i] (NULL ok) = min over
  * stance legs of n.f - F_min.  What a preview of a planned motion reports next to forces and torques

@@ -67,5 +67,5 @@ if __name__ == "__main__":
     print(build_host_demo(force=True, verbose=True))
     print(build_host_demo(force=True, verbose=True, which="qp_demo"))
     print(build_host_demo(force=True, verbose=True, which="swing_demo"))
-    for extra_demo in ("params_demo", "batch_demo", "nccl_demo", "threads_demo"):
+    for extra_demo in ("params_demo", "batch_demo", "nccl_demo", "threads_demo", "controller_demo"):
         print(build_host_demo(force=True, verbose=True, which=extra_demo))

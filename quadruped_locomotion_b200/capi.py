@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 
 import numpy as np
 
@@ -53,6 +54,8 @@ EXPORTS = (
     "qlb_default_swing_params", "qlb_set_limb_dynamics", "qlb_swing_leg_torques", "qlb_swing_leg_torques_host",
     "qlb_set_f32_core", "qlb_set_pipeline", "qlb_generate_states", "qlb_generate_states_f32", "qlb_solve_records", "qlb_solve_records_host", "qlb_stats_allreduce", "qlb_preview_plan_host", "qlb_params_set_key", "qlb_params_get_key", "qlb_params_num_keys", "qlb_params_key", "qlb_params_from_yaml", "qlb_swing_leg_torques_from_queue", "qlb_contact_fsm", "qlb_friction_margins", "qlb_leg_kinematics", "qlb_pack_robot_states", "qlb_feet_in_world", "qlb_qp_dense", "qlb_qp_dense_host", "qlb_batch_stats", "qlb_measure_fp64_peak", "qlb_launch_count", "qlb_strerror",
     "qlb_last_cuda_error", "qlb_abi_version",
+    "qlb_default_tick_params", "qlb_controller_create", "qlb_controller_destroy", "qlb_controller_reset",
+    "qlb_controller_update", "qlb_controller_update_host", "qlb_controller_get_state",
 )
 
 class LimbDynamics(C.Structure):
@@ -62,6 +65,10 @@ class LimbDynamics(C.Structure):
 
 class SwingParams(C.Structure):
     _fields_ = [("gravity", C.c_double * 3), ("acceleration_scale", C.c_double), ("kp", C.c_double * 3), ("kd", C.c_double * 3)]
+
+
+class TickParams(C.Structure):
+    _fields_ = [("period", C.c_double), ("effort_limit", C.c_double), ("swing", SwingParams)]
 
 
 # numpy mirror of qlb_robot_state_record (include/qlb.h)
@@ -154,6 +161,13 @@ def load() -> C.CDLL:
     lib.qlb_last_cuda_error.argtypes = [_vp]
     lib.qlb_last_cuda_error.restype = C.c_char_p
     lib.qlb_abi_version.restype = C.c_int
+    lib.qlb_default_tick_params.argtypes = [C.POINTER(TickParams)]
+    lib.qlb_controller_create.argtypes = [_vp, C.c_size_t, C.POINTER(TickParams), C.POINTER(_vp)]
+    lib.qlb_controller_destroy.argtypes = [_vp]
+    lib.qlb_controller_reset.argtypes = [_vp, _vp, _vp]
+    lib.qlb_controller_update.argtypes = [_vp] + [_vp] * 18
+    lib.qlb_controller_update_host.argtypes = [_vp] + [_vp] * 17
+    lib.qlb_controller_get_state.argtypes = [_vp, _vp, _vp, _vp]
     _lib = lib
     return lib
 
@@ -221,6 +235,8 @@ class Solver:
         self.device = int(device)
 
     def close(self):
+        for c in list(getattr(self, "_controllers", ())):   # a controller is destroyed before its context
+            c.close()
         if getattr(self, "_ctx", None) is not None and self._ctx.value:
             self.lib.qlb_destroy(self._ctx)
             self._ctx = _vp()
@@ -434,3 +450,68 @@ class Solver:
         net = np.zeros((6, B), dtype) if with_net else None
         self.solve_wrench_host(q, quat, wr, mask, mu, nr, grf, tau, flags, net)
         return dict(grf=grf, tau=tau, flags=flags, netwrench=net)
+
+
+def default_tick_params() -> TickParams:
+    p = TickParams()
+    if load().qlb_default_tick_params(C.byref(p)) != 0:
+        raise RuntimeError("qlb_default_tick_params failed")
+    return p
+
+
+class Controller:
+    """RosBalanceController::update for B robots: one update() per control tick, the limb states, joint efforts and
+    joint-velocity history of every robot kept on the device between ticks (include/qlb.h, qlb_controller_*).
+    Belongs to the Solver's context; Solver.close() closes it first."""
+
+    def __init__(self, solver: Solver, B: int, params: TickParams | None = None):
+        self.solver = solver
+        self.lib = solver.lib
+        self.B = int(B)
+        self._c = _vp()
+        rc = self.lib.qlb_controller_create(solver._ctx, self.B, C.byref(params) if params is not None else None, C.byref(self._c))
+        if rc != 0:
+            self._c = _vp()
+            solver._check(rc, "qlb_controller_create")
+        if not hasattr(solver, "_controllers"):
+            solver._controllers = weakref.WeakSet()
+        solver._controllers.add(self)
+
+    def close(self):
+        if getattr(self, "_c", None) is not None and self._c.value:
+            self.lib.qlb_controller_destroy(self._c)
+            self._c = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    # -- DEVICE pointers (torch CUDA tensors, SoA [C, B] contiguous float64; masks uint8 [B]; flags 32-bit [B])
+    def update(self, q, qd, pose, twist, tpose, ttwist, desired, contact, phase, command, flags, footstep=None, mu=None,
+               normals=None, ptarget=None, vtarget=None, grf=None, stream=None):
+        rc = self.lib.qlb_controller_update(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist),
+                                            _ptr(desired), _ptr(footstep), _ptr(contact), _ptr(phase), _ptr(mu), _ptr(normals),
+                                            _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags), _ptr(grf),
+                                            stream if stream is not None else None)
+        self.solver._check(rc, "qlb_controller_update")
+
+    def reset(self, mask=None, stream=None):
+        """RosBalanceController::starting for the robots with mask[i] != 0 (device uint8 [B]; None = all)."""
+        self.solver._check(self.lib.qlb_controller_reset(self._c, _ptr(mask), stream if stream is not None else None),
+                           "qlb_controller_reset")
+
+    def get_state(self, limb_state=None, efforts=None, stream=None):
+        """Device copies of the persistent state: limb_state uint8 [4, B], efforts float64 [12, B]."""
+        self.solver._check(self.lib.qlb_controller_get_state(self._c, _ptr(limb_state), _ptr(efforts),
+                                                             stream if stream is not None else None), "qlb_controller_get_state")
+
+    # -- HOST pointers (numpy arrays or pinned torch CPU tensors); synchronises
+    def update_host(self, q, qd, pose, twist, tpose, ttwist, desired, contact, phase, command, flags, footstep=None, mu=None,
+                    normals=None, ptarget=None, vtarget=None, grf=None):
+        rc = self.lib.qlb_controller_update_host(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist),
+                                                 _ptr(desired), _ptr(footstep), _ptr(contact), _ptr(phase), _ptr(mu),
+                                                 _ptr(normals), _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags),
+                                                 _ptr(grf))
+        self.solver._check(rc, "qlb_controller_update_host")

@@ -21,6 +21,7 @@
 #include "qlb_solve_fused.cuh"
 #include "qlb_solve_single.cuh"
 #include "qlb_swing.cuh"
+#include "qlb_tick.cuh"
 
 using namespace qlb;
 
@@ -1049,7 +1050,7 @@ int qlb_swing_leg_torques_from_queue(qlb_context* ctx, size_t B, const double* q
   DeviceGuard guard(ctx->device);
   SwingArgs a;
   std::memset(&a, 0, sizeof a);
-  a.B = B; a.q = q; a.qd = qd_back; a.qdd = nullptr; a.qd_front = qd_front; a.inv_window = 1.0 / (10.0 * period);
+  a.B = B; a.q = q; a.qd = qd_back; a.qdd = nullptr; a.qd_front = qd_front; a.ld_front = B; a.inv_window = 1.0 / (10.0 * period);
   a.ptarget = foot_target_position; a.vtarget = foot_target_velocity; a.tau = tau;
   for (int c = 0; c < 3; c++) { a.gravity[c] = params->gravity[c]; a.kp[c] = params->kp[c]; a.kd[c] = params->kd[c]; }
   a.acc_scale = params->acceleration_scale;
@@ -1477,6 +1478,241 @@ int qlb_measure_fp64_peak(qlb_context* ctx, double* tflops_out) {
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
   *tflops_out = best;
+  return QLB_OK;
+}
+
+}  // extern "C"
+
+// ---- the controller tick (qlb_controller_*)
+struct qlb_controller {
+  qlb_context* ctx = nullptr;
+  size_t B = 0;
+  qlb_tick_params p;
+  int head = 0;                 // ring slot of the next tick's sample
+  cudaEvent_t reset_done = nullptr;   // recorded by qlb_controller_reset: every update waits for it, whatever its stream
+  uint8_t* limb = nullptr;      // [4][B]
+  uint8_t* refill = nullptr;    // [B]
+  double* efforts = nullptr;    // [12][B]
+  double* ring = nullptr;       // [kTickRing][12][B]
+  uint8_t* stance = nullptr;    // scratch [B]: stance mask of the current tick
+  double* tau = nullptr;        // scratch [12][B]: torques of the solve
+  double* grf = nullptr;        // scratch [12][B]: forces of the solve when the caller passes none
+};
+
+namespace {
+
+// One tick for robots b0 .. b0 + n - 1 of the controller; the caller's arrays have row pitch n.
+int controller_tick(qlb_controller* c, size_t n, size_t b0, const double* q, const double* qd, const double* pose,
+                    const double* twist, const double* tpose, const double* ttwist, const uint8_t* desired,
+                    const uint8_t* footstep, const uint8_t* contact, const double* phase, const double* mu,
+                    const double* normals, const double* ptarget, const double* vtarget, double* command, uint32_t* flags,
+                    double* grf, cudaStream_t st) {
+  qlb_context* ctx = c->ctx;
+  const unsigned long long blocks_pro = ((unsigned long long)n + 255) / 256;
+  const unsigned long long blocks_epi = (4ull * n + 127) / 128;
+  if (blocks_epi > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
+  const size_t ld = c->B;
+  TickArgs a;
+  std::memset(&a, 0, sizeof a);
+  a.n = n; a.ld = ld; a.head = c->head;
+  a.desired = desired; a.footstep = footstep; a.contact = contact; a.phase = phase; a.qd = qd;
+  a.limb = c->limb + b0; a.refill = c->refill + b0; a.ring = c->ring + b0; a.stance = c->stance;
+  a.flags = flags; a.tau = c->tau; a.efforts = c->efforts + b0; a.command = command; a.limit = c->p.effort_limit;
+  SwingArgs& s = a.swing;
+  s.B = n; s.q = q; s.qd = qd;
+  s.qd_front = c->ring + (size_t)((c->head + 1) % kTickRing) * 12 * ld + b0; s.ld_front = ld;
+  s.inv_window = 1.0 / (10.0 * c->p.period);
+  s.ptarget = ptarget; s.vtarget = vtarget;
+  for (int k = 0; k < 3; k++) { s.gravity[k] = c->p.swing.gravity[k]; s.kp[k] = c->p.swing.kp[k]; s.kd[k] = c->p.swing.kd[k]; }
+  s.acc_scale = c->p.swing.acceleration_scale;
+  s.dyn = ctx->d_limb; s.model = ctx->d_model;
+  QLB_CUDA(ctx, cudaStreamWaitEvent(st, c->reset_done, 0));
+  qlb_tick_prologue_kernel<<<(unsigned)blocks_pro, 256, 0, st>>>(a);
+  QLB_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  const int rc = solve_state_t<double>(ctx, n, q, pose, twist, tpose, ttwist, c->stance, mu, normals, grf ? grf : c->grf, c->tau,
+                                       flags, nullptr, nullptr, st);
+  if (rc != QLB_OK) return rc;
+  qlb_tick_epilogue_kernel<<<(unsigned)blocks_epi, 128, 0, st>>>(a);
+  QLB_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  return QLB_OK;
+}
+
+bool controller_ready(const qlb_controller* c) { return c && c->ctx && c->ctx->have_limb; }
+
+}  // namespace
+
+extern "C" {
+
+int qlb_default_tick_params(qlb_tick_params* p) {
+  if (!p) return QLB_ERR_INVALID_ARGUMENT;
+  std::memset(p, 0, sizeof *p);
+  p->period = 0.0025;        // 400 Hz (balance_controller_manager.cpp:48,70)
+  p->effort_limit = 300.0;   // RBC.cpp:450-454
+  return qlb_default_swing_params(&p->swing);
+}
+
+int qlb_controller_create(qlb_context* ctx, size_t B, const qlb_tick_params* params, qlb_controller** out) {
+  static_assert(sizeof(qlb_tick_params) == 96, "qlb_tick_params layout is part of the ABI");
+  if (!out) return QLB_ERR_INVALID_ARGUMENT;
+  *out = nullptr;
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
+    cudaGetLastError();
+    return QLB_ERR_CUDA;
+  }
+  if (!ctx) return QLB_ERR_NOT_INITIALISED;
+  qlb_tick_params defaults;
+  qlb_default_tick_params(&defaults);
+  const qlb_tick_params* p = params ? params : &defaults;
+  if (B == 0 || !(p->period > 0.0) || !std::isfinite(p->period) || !(p->effort_limit >= 0.0) || !std::isfinite(p->effort_limit))
+    return QLB_ERR_INVALID_ARGUMENT;
+  if (B > 0xFFFFFFF0ull) return QLB_ERR_BATCH_TOO_LARGE;
+  QLB_GUARD(ctx);
+  DeviceGuard guard(ctx->device);
+  qlb_controller* c = new (std::nothrow) qlb_controller();
+  if (!c) return QLB_ERR_ALLOC;
+  c->ctx = ctx; c->B = B; c->p = *p;
+  if (cudaMalloc(&c->limb, 4 * B) != cudaSuccess || cudaMalloc(&c->refill, B) != cudaSuccess ||
+      cudaMalloc(&c->stance, B) != cudaSuccess || cudaMalloc(&c->efforts, 12 * B * sizeof(double)) != cudaSuccess ||
+      cudaMalloc(&c->ring, (size_t)kTickRing * 12 * B * sizeof(double)) != cudaSuccess ||
+      cudaMalloc(&c->tau, 12 * B * sizeof(double)) != cudaSuccess || cudaMalloc(&c->grf, 12 * B * sizeof(double)) != cudaSuccess) {
+    cudaGetLastError();
+    qlb_controller_destroy(c);
+    return QLB_ERR_ALLOC;
+  }
+  if (cudaEventCreateWithFlags(&c->reset_done, cudaEventDisableTiming) != cudaSuccess) {
+    const int rc = cuda_fail(ctx, cudaGetLastError(), "qlb_controller_create");
+    qlb_controller_destroy(c);
+    return rc;
+  }
+  static_assert(QLB_LIMB_INIT == 0, "limb states start as zero bytes");
+  if (cudaMemsetAsync(c->limb, 0, 4 * B, ctx->stream) != cudaSuccess || cudaMemsetAsync(c->refill, 1, B, ctx->stream) != cudaSuccess ||
+      cudaMemsetAsync(c->efforts, 0, 12 * B * sizeof(double), ctx->stream) != cudaSuccess ||
+      cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+    const int rc = cuda_fail(ctx, cudaGetLastError(), "qlb_controller_create");
+    qlb_controller_destroy(c);
+    return rc;
+  }
+  *out = c;
+  return QLB_OK;
+}
+
+int qlb_controller_destroy(qlb_controller* c) {
+  if (!c) return QLB_OK;
+  QLB_GUARD(c->ctx);
+  DeviceGuard guard(c->ctx->device);
+  cudaFree(c->limb); cudaFree(c->refill); cudaFree(c->stance); cudaFree(c->efforts); cudaFree(c->ring);
+  cudaFree(c->tau); cudaFree(c->grf);
+  if (c->reset_done) cudaEventDestroy(c->reset_done);
+  cudaGetLastError();
+  delete c;
+  return QLB_OK;
+}
+
+int qlb_controller_reset(qlb_controller* c, const uint8_t* reset_mask, void* stream) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  DeviceGuard guard(c->ctx->device);
+  const unsigned long long blocks = ((unsigned long long)c->B + 255) / 256;
+  qlb_tick_reset_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(c->B, reset_mask, c->limb, c->efforts,
+                                                                                         c->refill);
+  QLB_CUDA(c->ctx, cudaGetLastError());
+  c->ctx->launches++;
+  QLB_CUDA(c->ctx, cudaEventRecord(c->reset_done, static_cast<cudaStream_t>(stream)));
+  return QLB_OK;
+}
+
+int qlb_controller_update(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
+                          const double* base_twist, const double* target_pose, const double* target_twist,
+                          const uint8_t* desired_stance_mask, const uint8_t* footstep_mask, const uint8_t* contact_mask,
+                          const double* phase, const double* mu, const double* normals_world,
+                          const double* foot_target_position, const double* foot_target_velocity, double* command,
+                          uint32_t* flags, double* grf, void* stream) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
+  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
+      !phase || !command || !flags)
+    return QLB_ERR_INVALID_ARGUMENT;
+  DeviceGuard guard(c->ctx->device);
+  const int rc = controller_tick(c, c->B, 0, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                 footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                 foot_target_velocity, command, flags, grf, static_cast<cudaStream_t>(stream));
+  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
+  return rc;
+}
+
+// HOST pointers: chunks of the context's staging capacity, one after the other on the context stream; synchronises.
+int qlb_controller_update_host(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
+                               const double* base_twist, const double* target_pose, const double* target_twist,
+                               const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
+                               const uint8_t* contact_mask, const double* phase, const double* mu,
+                               const double* normals_world, const double* foot_target_position,
+                               const double* foot_target_velocity, double* command, uint32_t* flags, double* grf) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;
+  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
+      !phase || !command || !flags)
+    return QLB_ERR_INVALID_ARGUMENT;
+  qlb_context* ctx = c->ctx;
+  DeviceGuard guard(ctx->device);
+  int rc = ensure_capacity(ctx, c->B);
+  if (rc != QLB_OK) return rc;
+  const size_t B = c->B, cap = ctx->cap;
+  cudaStream_t st = ctx->stream;
+  // inputs: 94 rows in the input staging (kPipe * 54 rows of cap), outputs 24 rows, the three masks one row each
+  constexpr int kIn = 11, kOut = 2;
+  const double* src[kIn] = {q, qd, base_pose, base_twist, target_pose, target_twist, phase, mu, normals_world,
+                            foot_target_position, foot_target_velocity};
+  const int rows[kIn] = {12, 12, 7, 6, 7, 6, 4, 4, 12, 12, 12};
+  static_assert(kPipe * kHostInRows >= 94 && kPipe * kHostOutRows >= 24 && kPipe >= 3, "staging too small for a tick");
+  const uint8_t* msrc[3] = {desired_stance_mask, footstep_mask, contact_mask};
+  double* dst_out[kOut] = {command, grf};
+  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap) {
+    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
+    const double* din[kIn];
+    size_t off = 0;
+    for (int k = 0; k < kIn && rc == QLB_OK; k++) {
+      din[k] = src[k] ? ctx->d_in + off : nullptr;
+      if (src[k] && cudaMemcpy2DAsync(ctx->d_in + off, n * sizeof(double), src[k] + b0, B * sizeof(double), n * sizeof(double),
+                                      rows[k], cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+      off += (size_t)rows[k] * cap;
+    }
+    const uint8_t* dmask[3];
+    for (int k = 0; k < 3 && rc == QLB_OK; k++) {
+      dmask[k] = msrc[k] ? ctx->d_mask + (size_t)k * cap : nullptr;
+      if (msrc[k] && cudaMemcpyAsync(ctx->d_mask + (size_t)k * cap, msrc[k] + b0, n, cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+    }
+    if (rc != QLB_OK) break;
+    double* dout[kOut] = {ctx->d_out, ctx->d_out + 12 * cap};
+    rc = controller_tick(c, n, b0, din[0], din[1], din[2], din[3], din[4], din[5], dmask[0], dmask[1], dmask[2], din[6], din[7],
+                         din[8], din[9], din[10], dout[0], ctx->d_flags, dout[1], st);
+    for (int k = 0; k < kOut && rc == QLB_OK; k++)
+      if (dst_out[k] && cudaMemcpy2DAsync(dst_out[k] + b0, B * sizeof(double), dout[k], n * sizeof(double), n * sizeof(double), 12,
+                                          cudaMemcpyDeviceToHost, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+    if (rc == QLB_OK && cudaMemcpyAsync(flags + b0, ctx->d_flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess)
+      rc = QLB_ERR_CUDA;
+  }
+  // also on failure: no copy may still be reading or writing the caller's buffers when the call returns
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
+  if (rc == QLB_ERR_CUDA) return cuda_fail(ctx, cudaGetLastError(), "qlb_controller_update_host");
+  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
+  return rc;
+}
+
+int qlb_controller_get_state(const qlb_controller* c, uint8_t* limb_state, double* efforts, void* stream) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  DeviceGuard guard(c->ctx->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (limb_state) QLB_CUDA(c->ctx, cudaMemcpyAsync(limb_state, c->limb, 4 * c->B, cudaMemcpyDeviceToDevice, st));
+  if (efforts) QLB_CUDA(c->ctx, cudaMemcpyAsync(efforts, c->efforts, 12 * c->B * sizeof(double), cudaMemcpyDeviceToDevice, st));
   return QLB_OK;
 }
 

@@ -260,19 +260,17 @@ __global__ void __launch_bounds__(256) qlb_stats_kernel(unsigned long long B, co
 //   stance    [B] out: bit k = leg k is a support leg for the force distribution
 // (The reference advances its limb index only at the end of the loop body, so a `continue` makes the next foot
 // overwrite the same limb; the per-limb rules below are the evident intent.)
-__global__ void __launch_bounds__(256) qlb_contact_fsm_kernel(unsigned long long B, const uint8_t* __restrict__ desired,
-                                                              const uint8_t* __restrict__ footstep, const uint8_t* __restrict__ contact,
-                                                              const double* __restrict__ phase, uint8_t* __restrict__ limb_state,
-                                                              uint8_t* __restrict__ stance) {
-  const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= B) return;
-  const unsigned des = desired[i], fs = footstep ? footstep[i] : 0xFu, con = contact[i];
+// One robot i: phase has row pitch ld_phase, limb_state row pitch ld_limb (the controller tick keeps its limb states
+// in arrays of its own batch size).  Returns the stance mask.
+__device__ __forceinline__ unsigned contact_fsm_robot(unsigned long long i, unsigned des, unsigned fs, unsigned con,
+                                                      const double* __restrict__ phase, unsigned long long ld_phase,
+                                                      uint8_t* __restrict__ limb_state, unsigned long long ld_limb) {
   unsigned mask = 0u;
 #pragma unroll
   for (int k = 0; k < 4; k++) {
     const bool d = (des >> k) & 1u, f = (fs >> k) & 1u, c = (con >> k) & 1u;
-    const double ph = phase[(size_t)k * B + i];
-    unsigned st = limb_state[(size_t)k * B + i];
+    const double ph = phase[(size_t)k * ld_phase + i];
+    unsigned st = limb_state[(size_t)k * ld_limb + i];
     if (!d) {
       st = QLB_LIMB_SWING_NORMAL;
       if (f) {
@@ -288,10 +286,20 @@ __global__ void __launch_bounds__(256) qlb_contact_fsm_kernel(unsigned long long
         if (ph > 0.5 && !c) st = QLB_LIMB_STANCE_LOST_CONTACT;
       }
     }
-    limb_state[(size_t)k * B + i] = (uint8_t)st;
+    limb_state[(size_t)k * ld_limb + i] = (uint8_t)st;
     const bool support = st == QLB_LIMB_STANCE_NORMAL || st == QLB_LIMB_SWING_EARLY_TOUCHDOWN || st == QLB_LIMB_INIT;
     mask |= (support ? 1u : 0u) << k;
   }
+  return mask;
+}
+
+__global__ void __launch_bounds__(256) qlb_contact_fsm_kernel(unsigned long long B, const uint8_t* __restrict__ desired,
+                                                              const uint8_t* __restrict__ footstep, const uint8_t* __restrict__ contact,
+                                                              const double* __restrict__ phase, uint8_t* __restrict__ limb_state,
+                                                              uint8_t* __restrict__ stance) {
+  const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B) return;
+  const unsigned mask = contact_fsm_robot(i, desired[i], footstep ? footstep[i] : 0xFu, contact[i], phase, B, limb_state, B);
   if (stance) stance[i] = (uint8_t)mask;
 }
 

@@ -446,4 +446,88 @@ class MyRobotSolver {
   bool loaded_ = false;
 };
 
+// ---------------------------------------------------------------- RosBalanceController
+// The whole controller tick of one robot (ros_balance_controller.cpp:198-716 update, starting) over
+// qlb_controller_update_host with B = 1: contact state machine, virtual model + force distribution for the stance legs,
+// swing-leg dynamics with the joint-velocity history, stale efforts on a failed solve and the +-300 N m command clamp.
+// Measured and desired base state, joint positions and surface normals come from the shared State; the per-leg plan and
+// contact inputs, the joint velocities and the swing targets are set on the controller.  The joint efforts that survive
+// between ticks stay on the device (qlb_controller_get_state); update() returns the clamped command.
+class RosBalanceController {
+ public:
+  RosBalanceController(std::shared_ptr<Device> device, std::shared_ptr<State> state,
+                       const qlb_limb_dynamics* limbs = QLB_LIMB_DYNAMICS_QUADRUPED_MODEL)
+      : device_(std::move(device)), robot_state_(std::move(state)), limbs_(limbs) {
+    qlb_default_tick_params(&params_);
+    phase_.fill(0.0);
+  }
+  ~RosBalanceController() { qlb_controller_destroy(ctrl_); }
+  RosBalanceController(const RosBalanceController&) = delete;
+  RosBalanceController& operator=(const RosBalanceController&) = delete;
+
+  qlb_tick_params& params() { return params_; }   // period, effort limit and swing gains; read by init()
+  // ros_balance_controller.cpp init(): limb models and the controller state for one robot
+  bool init() {
+    if (ctrl_) return false;
+    if (qlb_set_limb_dynamics(device_->ctx(), limbs_) != QLB_OK) return false;
+    return qlb_controller_create(device_->ctx(), 1, &params_, &ctrl_) == QLB_OK;
+  }
+  // RosBalanceController::starting: limb states INIT, efforts zero, velocity history restarted
+  bool starting() { return ctrl_ && qlb_controller_reset(ctrl_, nullptr, nullptr) == QLB_OK; }
+
+  // limbs_desired_state_ / is_footstep_ / FootContacts.is_contact / st_phase, sw_phase of one leg
+  void setLimbInput(LimbEnum limb, bool desired_stance, bool is_footstep, bool is_contact, double phase) {
+    const int l = static_cast<int>(limb);
+    const uint8_t bit = static_cast<uint8_t>(1u << l);
+    desired_ = desired_stance ? (desired_ | bit) : (desired_ & ~bit);
+    footstep_ = is_footstep ? (footstep_ | bit) : (footstep_ & ~bit);
+    contact_ = is_contact ? (contact_ | bit) : (contact_ & ~bit);
+    phase_[l] = phase;
+  }
+  void setJointVelocities(const JointEfforts& qd) { qd_ = qd; }   // measured joint velocities, LF..LH x 3
+  void setSwingTarget(LimbEnum limb, const Position& position, const LinearVelocity& velocity) {   // base frame
+    const int l = static_cast<int>(limb);
+    for (int i = 0; i < 3; i++) { ptarget_[3 * l + i] = position[i]; vtarget_[3 * l + i] = velocity[i]; }
+  }
+
+  // RosBalanceController::update(time, period).  The period is fixed when the controller is created (the velocity
+  // history spans ten of them): a different one is refused.
+  bool update(double /*time*/, double period) {
+    if (!ctrl_ || period != params_.period) return false;
+    const State& s = *robot_state_;
+    double q[12], qd[12], pose[7], twist[6], tpose[7], ttwist[6], normals[12], phase[4];
+    for (int i = 0; i < 12; i++) { q[i] = s.getJointPositionFeedback()[i]; qd[i] = qd_[i]; }
+    for (int a = 0; a < 3; a++) {
+      pose[a] = s.getPositionWorldToBaseInWorldFrame()[a]; tpose[a] = s.getTargetPositionWorldToBaseInWorldFrame()[a];
+      twist[a] = s.getLinearVelocityBaseInWorldFrame()[a]; twist[3 + a] = s.getAngularVelocityBaseInBaseFrame()[a];
+      ttwist[a] = s.getTargetLinearVelocityBaseInWorldFrame()[a]; ttwist[3 + a] = s.getTargetAngularVelocityBaseInBaseFrame()[a];
+    }
+    for (int i = 0; i < 4; i++) { pose[3 + i] = s.getOrientationBaseToWorld()[i]; tpose[3 + i] = s.getTargetOrientationBaseToWorld()[i]; }
+    for (int l = 0; l < 4; l++) {
+      phase[l] = phase_[l];
+      for (int a = 0; a < 3; a++) normals[3 * l + a] = s.getSurfaceNormal(static_cast<LimbEnum>(l))[a];
+    }
+    return qlb_controller_update_host(ctrl_, q, qd, pose, twist, tpose, ttwist, &desired_, &footstep_, &contact_, phase, nullptr,
+                                      normals, ptarget_, vtarget_, command_.data(), &flags_, grf_) == QLB_OK;
+  }
+  const JointEfforts& getCommand() const { return command_; }   // clamped to +-effort_limit
+  uint32_t getFlags() const { return flags_; }                  // result word of the tick's solve
+  Force getGroundReactionForce(LimbEnum limb) const {
+    const int l = static_cast<int>(limb);
+    return {{grf_[3 * l], grf_[3 * l + 1], grf_[3 * l + 2]}};
+  }
+
+ private:
+  std::shared_ptr<Device> device_;
+  std::shared_ptr<State> robot_state_;
+  const qlb_limb_dynamics* limbs_;
+  qlb_tick_params params_;
+  qlb_controller* ctrl_ = nullptr;
+  uint8_t desired_ = 0xF, footstep_ = 0xF, contact_ = 0xF;
+  std::array<double, 4> phase_;
+  JointEfforts qd_{}, command_{};
+  double ptarget_[12] = {0}, vtarget_[12] = {0}, grf_[12] = {0};
+  uint32_t flags_ = 0;
+};
+
 }  // namespace qlb_host
