@@ -455,6 +455,36 @@ int qlb_controller_update_host(qlb_controller* c, const double* q, const double*
                                const uint8_t* contact_mask, const double* phase, const double* mu,
                                const double* normals_world, const double* foot_target_position,
                                const double* foot_target_velocity, double* command, uint32_t* flags, double* grf);
+/* FP32 twins of the tick, for a caller that keeps its state in float: the same arguments, NULL rules, errors, ordering
+ * and launches as above, with float arrays.  They act on the same controller, whose state stays FP64 (limb states,
+ * efforts, the ring of qd samples: a float sample is stored exactly), so the FP64 and FP32 updates may be mixed from
+ * tick to tick; qlb_controller_get_state is unchanged.
+ *   contact state machine: the float phase is widened to double before the comparisons, so the limb states are those
+ *     of the FP64 tick on the same values, bit for bit
+ *   stance legs: qlb_solve_state_f32 (the solver core follows qlb_set_f32_core; the default FP64 core)
+ *   swing legs: FP32 arithmetic on FP32 copies of the limb tables and the kinematic model; qdd differenced in FP32
+ *     from the float sample and the oldest ring slot rounded to float (exact when only FP32 updates wrote it)
+ *   command: the FP64 efforts clamped to +-effort_limit in double, then rounded to float
+ * Stale rows, the clamp and the reset behave as in FP64.  One difference: FP32 overflows earlier, so a huge but finite
+ * qd can make a swing row stale (non-finite FP32 torque) where the FP64 tick would not.
+ * STATED TOLERANCE against the FP64 tick on the same values widened to double (tests/test_controller_f32.py, 40-tick
+ * trot): limb states and the status and contact bits of flags exact; active-row bits equal on >= 99.9 % of robot-ticks;
+ * stance rows of command and efforts within 1e-3 per robot (scale max(1, |x|_inf)), grf within 5e-4 (the bars of the
+ * solve twin); swing rows within 1e-4.  Measured on one B200 (1000 W power limit, 4099 robots over 40 ticks): limb states,
+ * status and contact bits exact; active-row bits equal on every robot-tick; stance rows 1.1e-4, grf 7.2e-5, swing rows
+ * 4.4e-6.  Speed on the same card: 2^20 robots 1.52 ms per tick against 1.86 ms for the FP64 tick (DESIGN.md section 5). */
+int qlb_controller_update_f32(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
+                              const float* base_twist, const float* target_pose, const float* target_twist,
+                              const uint8_t* desired_stance_mask, const uint8_t* footstep_mask, const uint8_t* contact_mask,
+                              const float* phase, const float* mu, const float* normals_world,
+                              const float* foot_target_position, const float* foot_target_velocity, float* command,
+                              uint32_t* flags, float* grf, void* stream);
+int qlb_controller_update_f32_host(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
+                                   const float* base_twist, const float* target_pose, const float* target_twist,
+                                   const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
+                                   const uint8_t* contact_mask, const float* phase, const float* mu,
+                                   const float* normals_world, const float* foot_target_position,
+                                   const float* foot_target_velocity, float* command, uint32_t* flags, float* grf);
 /* DEVICE copies of the persistent state, asynchronous on `stream`: limb_state[4][B], efforts[12][B] (either NULL ok). */
 int qlb_controller_get_state(const qlb_controller* c, uint8_t* limb_state, double* efforts, void* stream);
 

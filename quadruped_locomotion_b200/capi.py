@@ -56,6 +56,7 @@ EXPORTS = (
     "qlb_last_cuda_error", "qlb_abi_version",
     "qlb_default_tick_params", "qlb_controller_create", "qlb_controller_destroy", "qlb_controller_reset",
     "qlb_controller_update", "qlb_controller_update_host", "qlb_controller_get_state",
+    "qlb_controller_update_f32", "qlb_controller_update_f32_host",
 )
 
 class LimbDynamics(C.Structure):
@@ -167,6 +168,8 @@ def load() -> C.CDLL:
     lib.qlb_controller_reset.argtypes = [_vp, _vp, _vp]
     lib.qlb_controller_update.argtypes = [_vp] + [_vp] * 18
     lib.qlb_controller_update_host.argtypes = [_vp] + [_vp] * 17
+    lib.qlb_controller_update_f32.argtypes = [_vp] + [_vp] * 18
+    lib.qlb_controller_update_f32_host.argtypes = [_vp] + [_vp] * 17
     lib.qlb_controller_get_state.argtypes = [_vp, _vp, _vp, _vp]
     _lib = lib
     return lib
@@ -488,13 +491,26 @@ class Controller:
         except Exception:
             pass
 
-    # -- DEVICE pointers (torch CUDA tensors, SoA [C, B] contiguous float64; masks uint8 [B]; flags 32-bit [B])
+    @staticmethod
+    def _pick(fn64, fn32, arrays):
+        """The FP64 entry point, or its _f32 twin when q is float32.  Every floating-point array of the call must have
+        the dtype of q: the library reads each array as that type."""
+        dtypes = {str(a.dtype).split(".")[-1] for a in arrays if a is not None}
+        if len(dtypes) > 1:
+            raise TypeError(f"controller update: floating-point arrays of mixed dtypes {sorted(dtypes)}; "
+                            "use float64 throughout, or float32 throughout for the _f32 twin")
+        return fn32 if _is_f32(arrays[0]) else fn64
+
+    # -- DEVICE pointers (torch CUDA tensors, SoA [C, B] contiguous float64, or float32 throughout for the _f32 twin;
+    #    masks uint8 [B]; flags 32-bit [B])
     def update(self, q, qd, pose, twist, tpose, ttwist, desired, contact, phase, command, flags, footstep=None, mu=None,
                normals=None, ptarget=None, vtarget=None, grf=None, stream=None):
-        rc = self.lib.qlb_controller_update(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist),
-                                            _ptr(desired), _ptr(footstep), _ptr(contact), _ptr(phase), _ptr(mu), _ptr(normals),
-                                            _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags), _ptr(grf),
-                                            stream if stream is not None else None)
+        fn = self._pick(self.lib.qlb_controller_update, self.lib.qlb_controller_update_f32,
+                        (q, qd, pose, twist, tpose, ttwist, phase, mu, normals, ptarget, vtarget, command, grf))
+        rc = fn(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist),
+                _ptr(desired), _ptr(footstep), _ptr(contact), _ptr(phase), _ptr(mu), _ptr(normals),
+                _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags), _ptr(grf),
+                stream if stream is not None else None)
         self.solver._check(rc, "qlb_controller_update")
 
     def reset(self, mask=None, stream=None):
@@ -510,8 +526,9 @@ class Controller:
     # -- HOST pointers (numpy arrays or pinned torch CPU tensors); synchronises
     def update_host(self, q, qd, pose, twist, tpose, ttwist, desired, contact, phase, command, flags, footstep=None, mu=None,
                     normals=None, ptarget=None, vtarget=None, grf=None):
-        rc = self.lib.qlb_controller_update_host(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist),
-                                                 _ptr(desired), _ptr(footstep), _ptr(contact), _ptr(phase), _ptr(mu),
-                                                 _ptr(normals), _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags),
-                                                 _ptr(grf))
+        fn = self._pick(self.lib.qlb_controller_update_host, self.lib.qlb_controller_update_f32_host,
+                        (q, qd, pose, twist, tpose, ttwist, phase, mu, normals, ptarget, vtarget, command, grf))
+        rc = fn(self._c, _ptr(q), _ptr(qd), _ptr(pose), _ptr(twist), _ptr(tpose), _ptr(ttwist), _ptr(desired), _ptr(footstep),
+                _ptr(contact), _ptr(phase), _ptr(mu), _ptr(normals), _ptr(ptarget), _ptr(vtarget), _ptr(command), _ptr(flags),
+                _ptr(grf))
         self.solver._check(rc, "qlb_controller_update_host")

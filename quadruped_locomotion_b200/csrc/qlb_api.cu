@@ -40,6 +40,7 @@ struct qlb_context {
   DeviceModel* d_model = nullptr;
   DeviceParams* d_params = nullptr;
   DeviceLimbDynamics* d_limb = nullptr;        // qlb_set_limb_dynamics
+  DeviceLimbDynamicsT<float>* d_limb_f = nullptr;   // its FP32 copy (swing legs of qlb_controller_update_f32)
   bool have_limb = false;
   DeviceModelT<float>* d_model_f = nullptr;    // FP32 copies for the _f32 entry points
   DeviceParamsT<float>* d_params_f = nullptr;
@@ -679,7 +680,7 @@ int qlb_destroy(qlb_context* ctx) {
   for (int i = 0; i < kPipe; i++)
     if (ctx->pipe[i]) { cudaStreamSynchronize(ctx->pipe[i]); cudaStreamDestroy(ctx->pipe[i]); }
   cudaFree(ctx->d_model); cudaFree(ctx->d_params); cudaFree(ctx->d_counter); cudaFree(ctx->d_stats);
-  cudaFree(ctx->d_model_f); cudaFree(ctx->d_params_f); cudaFree(ctx->d_limb);
+  cudaFree(ctx->d_model_f); cudaFree(ctx->d_params_f); cudaFree(ctx->d_limb); cudaFree(ctx->d_limb_f);
   cudaFree(ctx->d_in); cudaFree(ctx->d_out); cudaFree(ctx->d_mask); cudaFree(ctx->d_flags); cudaFree(ctx->d_rec); cudaFree(ctx->d_qp); cudaFree(ctx->d_prev);
   for (int i = 0; i < 8; i++) cudaFree(ctx->d_list[i]);
   for (int i = 0; i < 8; i++)
@@ -737,11 +738,13 @@ namespace {
 template <typename T> struct Typed;
 template <> struct Typed<double> {
   static const DeviceModel* model(const qlb_context* c) { return c->d_model; }
+  static const DeviceLimbDynamics* limb(const qlb_context* c) { return c->d_limb; }
   static const DeviceParams* params(const qlb_context* c) { return c->d_params; }
   template <int MODE> static int launch(qlb_context* c, SolveArgs& a, cudaStream_t st) { return launch_solve<MODE>(c, a, st); }
 };
 template <> struct Typed<float> {
   static const DeviceModelT<float>* model(const qlb_context* c) { return c->d_model_f; }
+  static const DeviceLimbDynamicsT<float>* limb(const qlb_context* c) { return c->d_limb_f; }
   static const DeviceParamsT<float>* params(const qlb_context* c) { return c->d_params_f; }
   template <int MODE> static int launch(qlb_context* c, SolveArgsT<float>& a, cudaStream_t st) { return launch_solve_f32<MODE>(c, a, st); }
 };
@@ -1008,9 +1011,17 @@ int qlb_set_limb_dynamics(qlb_context* ctx, const qlb_limb_dynamics legs[QLB_NUM
       h.mass[l][j] = legs[l].body_mass[j];
       for (int a = 0; a < 6; a++) h.inertia[l][j][a] = legs[l].body_inertia[j][a];
     }
+  // FP32 copy: same fields, rounded once on the host (as narrow_model)
+  DeviceLimbDynamicsT<float> hf;
+  static_assert(sizeof hf * 2 == sizeof h, "the FP32 copy narrows every field");
+  const double* src = reinterpret_cast<const double*>(&h);
+  float* dst = reinterpret_cast<float*>(&hf);
+  for (size_t i = 0; i < sizeof h / sizeof(double); i++) dst[i] = (float)src[i];
   if (!ctx->d_limb && cudaMalloc(&ctx->d_limb, sizeof h) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
+  if (!ctx->d_limb_f && cudaMalloc(&ctx->d_limb_f, sizeof hf) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
   QLB_CUDA(ctx, cudaDeviceSynchronize());
   QLB_CUDA(ctx, cudaMemcpy(ctx->d_limb, &h, sizeof h, cudaMemcpyHostToDevice));
+  QLB_CUDA(ctx, cudaMemcpy(ctx->d_limb_f, &hf, sizeof hf, cudaMemcpyHostToDevice));
   ctx->have_limb = true;
   return QLB_OK;
 }
@@ -1501,45 +1512,133 @@ struct qlb_controller {
 
 namespace {
 
-// One tick for robots b0 .. b0 + n - 1 of the controller; the caller's arrays have row pitch n.
-int controller_tick(qlb_controller* c, size_t n, size_t b0, const double* q, const double* qd, const double* pose,
-                    const double* twist, const double* tpose, const double* ttwist, const uint8_t* desired,
-                    const uint8_t* footstep, const uint8_t* contact, const double* phase, const double* mu,
-                    const double* normals, const double* ptarget, const double* vtarget, double* command, uint32_t* flags,
-                    double* grf, cudaStream_t st) {
+// One tick for robots b0 .. b0 + n - 1 of the controller; the caller's arrays have row pitch n.  T = float: the
+// swing legs in FP32 on the FP32 tables, the stance legs by solve_state_t<float> on the scratch reinterpreted as float
+// (12 n doubles hold 12 n floats); the solver core follows the context's qlb_set_f32_core.
+template <typename T>
+int controller_tick(qlb_controller* c, size_t n, size_t b0, const T* q, const T* qd, const T* pose, const T* twist,
+                    const T* tpose, const T* ttwist, const uint8_t* desired, const uint8_t* footstep, const uint8_t* contact,
+                    const T* phase, const T* mu, const T* normals, const T* ptarget, const T* vtarget, T* command,
+                    uint32_t* flags, T* grf, cudaStream_t st) {
   qlb_context* ctx = c->ctx;
   const unsigned long long blocks_pro = ((unsigned long long)n + 255) / 256;
   const unsigned long long blocks_epi = (4ull * n + 127) / 128;
   if (blocks_epi > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
   const size_t ld = c->B;
-  TickArgs a;
+  T* tau = reinterpret_cast<T*>(c->tau);
+  TickArgsT<T> a;
   std::memset(&a, 0, sizeof a);
   a.n = n; a.ld = ld; a.head = c->head;
   a.desired = desired; a.footstep = footstep; a.contact = contact; a.phase = phase; a.qd = qd;
   a.limb = c->limb + b0; a.refill = c->refill + b0; a.ring = c->ring + b0; a.stance = c->stance;
-  a.flags = flags; a.tau = c->tau; a.efforts = c->efforts + b0; a.command = command; a.limit = c->p.effort_limit;
-  SwingArgs& s = a.swing;
+  a.flags = flags; a.tau = tau; a.efforts = c->efforts + b0; a.command = command; a.limit = c->p.effort_limit;
+  SwingArgsT<T>& s = a.swing;
   s.B = n; s.q = q; s.qd = qd;
   s.qd_front = c->ring + (size_t)((c->head + 1) % kTickRing) * 12 * ld + b0; s.ld_front = ld;
-  s.inv_window = 1.0 / (10.0 * c->p.period);
+  s.inv_window = (T)(1.0 / (10.0 * c->p.period));
   s.ptarget = ptarget; s.vtarget = vtarget;
-  for (int k = 0; k < 3; k++) { s.gravity[k] = c->p.swing.gravity[k]; s.kp[k] = c->p.swing.kp[k]; s.kd[k] = c->p.swing.kd[k]; }
-  s.acc_scale = c->p.swing.acceleration_scale;
-  s.dyn = ctx->d_limb; s.model = ctx->d_model;
+  for (int k = 0; k < 3; k++) { s.gravity[k] = (T)c->p.swing.gravity[k]; s.kp[k] = (T)c->p.swing.kp[k]; s.kd[k] = (T)c->p.swing.kd[k]; }
+  s.acc_scale = (T)c->p.swing.acceleration_scale;
+  s.dyn = Typed<T>::limb(ctx); s.model = Typed<T>::model(ctx);
   QLB_CUDA(ctx, cudaStreamWaitEvent(st, c->reset_done, 0));
-  qlb_tick_prologue_kernel<<<(unsigned)blocks_pro, 256, 0, st>>>(a);
+  qlb_tick_prologue_kernel<T><<<(unsigned)blocks_pro, 256, 0, st>>>(a);
   QLB_CUDA(ctx, cudaGetLastError());
   ctx->launches++;
-  const int rc = solve_state_t<double>(ctx, n, q, pose, twist, tpose, ttwist, c->stance, mu, normals, grf ? grf : c->grf, c->tau,
-                                       flags, nullptr, nullptr, st);
+  const int rc = solve_state_t<T>(ctx, n, q, pose, twist, tpose, ttwist, c->stance, mu, normals,
+                                  grf ? grf : reinterpret_cast<T*>(c->grf), tau, flags, nullptr, nullptr, st);
   if (rc != QLB_OK) return rc;
-  qlb_tick_epilogue_kernel<<<(unsigned)blocks_epi, 128, 0, st>>>(a);
+  qlb_tick_epilogue_kernel<T><<<(unsigned)blocks_epi, 128, 0, st>>>(a);
   QLB_CUDA(ctx, cudaGetLastError());
   ctx->launches++;
   return QLB_OK;
 }
 
 bool controller_ready(const qlb_controller* c) { return c && c->ctx && c->ctx->have_limb; }
+
+template <typename T>
+int controller_update_t(qlb_controller* c, const T* q, const T* qd, const T* base_pose, const T* base_twist,
+                        const T* target_pose, const T* target_twist, const uint8_t* desired_stance_mask,
+                        const uint8_t* footstep_mask, const uint8_t* contact_mask, const T* phase, const T* mu,
+                        const T* normals_world, const T* foot_target_position, const T* foot_target_velocity, T* command,
+                        uint32_t* flags, T* grf, void* stream) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
+  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
+      !phase || !command || !flags)
+    return QLB_ERR_INVALID_ARGUMENT;
+  DeviceGuard guard(c->ctx->device);
+  const int rc = controller_tick<T>(c, c->B, 0, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                    footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                    foot_target_velocity, command, flags, grf, static_cast<cudaStream_t>(stream));
+  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
+  return rc;
+}
+
+// HOST pointers: chunks of the context's staging capacity, one after the other on the context stream; synchronises.
+// The staging buffers are sized for FP64; the FP32 twin uses the same row offsets in float, i.e. the first half.
+template <typename T>
+int controller_update_host_t(qlb_controller* c, const T* q, const T* qd, const T* base_pose, const T* base_twist,
+                             const T* target_pose, const T* target_twist, const uint8_t* desired_stance_mask,
+                             const uint8_t* footstep_mask, const uint8_t* contact_mask, const T* phase, const T* mu,
+                             const T* normals_world, const T* foot_target_position, const T* foot_target_velocity,
+                             T* command, uint32_t* flags, T* grf) {
+  if (!c) return QLB_ERR_NOT_INITIALISED;
+  QLB_GUARD(c->ctx);
+  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;
+  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
+      !phase || !command || !flags)
+    return QLB_ERR_INVALID_ARGUMENT;
+  qlb_context* ctx = c->ctx;
+  DeviceGuard guard(ctx->device);
+  int rc = ensure_capacity(ctx, c->B);
+  if (rc != QLB_OK) return rc;
+  const size_t B = c->B, cap = ctx->cap;
+  cudaStream_t st = ctx->stream;
+  T* const d_in = reinterpret_cast<T*>(ctx->d_in);
+  T* const d_out = reinterpret_cast<T*>(ctx->d_out);
+  // inputs: 94 rows in the input staging (kPipe * 54 rows of cap), outputs 24 rows, the three masks one row each
+  constexpr int kIn = 11, kOut = 2;
+  const T* src[kIn] = {q, qd, base_pose, base_twist, target_pose, target_twist, phase, mu, normals_world,
+                       foot_target_position, foot_target_velocity};
+  const int rows[kIn] = {12, 12, 7, 6, 7, 6, 4, 4, 12, 12, 12};
+  static_assert(kPipe * kHostInRows >= 94 && kPipe * kHostOutRows >= 24 && kPipe >= 3, "staging too small for a tick");
+  const uint8_t* msrc[3] = {desired_stance_mask, footstep_mask, contact_mask};
+  T* dst_out[kOut] = {command, grf};
+  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap) {
+    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
+    const T* din[kIn];
+    size_t off = 0;
+    for (int k = 0; k < kIn && rc == QLB_OK; k++) {
+      din[k] = src[k] ? d_in + off : nullptr;
+      if (src[k] && cudaMemcpy2DAsync(d_in + off, n * sizeof(T), src[k] + b0, B * sizeof(T), n * sizeof(T), rows[k],
+                                      cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+      off += (size_t)rows[k] * cap;
+    }
+    const uint8_t* dmask[3];
+    for (int k = 0; k < 3 && rc == QLB_OK; k++) {
+      dmask[k] = msrc[k] ? ctx->d_mask + (size_t)k * cap : nullptr;
+      if (msrc[k] && cudaMemcpyAsync(ctx->d_mask + (size_t)k * cap, msrc[k] + b0, n, cudaMemcpyHostToDevice, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+    }
+    if (rc != QLB_OK) break;
+    T* dout[kOut] = {d_out, d_out + 12 * cap};
+    rc = controller_tick<T>(c, n, b0, din[0], din[1], din[2], din[3], din[4], din[5], dmask[0], dmask[1], dmask[2], din[6],
+                            din[7], din[8], din[9], din[10], dout[0], ctx->d_flags, dout[1], st);
+    for (int k = 0; k < kOut && rc == QLB_OK; k++)
+      if (dst_out[k] && cudaMemcpy2DAsync(dst_out[k] + b0, B * sizeof(T), dout[k], n * sizeof(T), n * sizeof(T), 12,
+                                          cudaMemcpyDeviceToHost, st) != cudaSuccess)
+        rc = QLB_ERR_CUDA;
+    if (rc == QLB_OK && cudaMemcpyAsync(flags + b0, ctx->d_flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess)
+      rc = QLB_ERR_CUDA;
+  }
+  // also on failure: no copy may still be reading or writing the caller's buffers when the call returns
+  if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
+  if (rc == QLB_ERR_CUDA) return cuda_fail(ctx, cudaGetLastError(), "qlb_controller_update_host");
+  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
+  return rc;
+}
 
 }  // namespace
 
@@ -1630,80 +1729,39 @@ int qlb_controller_update(qlb_controller* c, const double* q, const double* qd, 
                           const double* phase, const double* mu, const double* normals_world,
                           const double* foot_target_position, const double* foot_target_velocity, double* command,
                           uint32_t* flags, double* grf, void* stream) {
-  if (!c) return QLB_ERR_NOT_INITIALISED;
-  QLB_GUARD(c->ctx);
-  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
-  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
-      !phase || !command || !flags)
-    return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(c->ctx->device);
-  const int rc = controller_tick(c, c->B, 0, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
-                                 footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                 foot_target_velocity, command, flags, grf, static_cast<cudaStream_t>(stream));
-  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
-  return rc;
+  return controller_update_t<double>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                     footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                     foot_target_velocity, command, flags, grf, stream);
 }
-
-// HOST pointers: chunks of the context's staging capacity, one after the other on the context stream; synchronises.
+int qlb_controller_update_f32(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
+                              const float* base_twist, const float* target_pose, const float* target_twist,
+                              const uint8_t* desired_stance_mask, const uint8_t* footstep_mask, const uint8_t* contact_mask,
+                              const float* phase, const float* mu, const float* normals_world,
+                              const float* foot_target_position, const float* foot_target_velocity, float* command,
+                              uint32_t* flags, float* grf, void* stream) {
+  return controller_update_t<float>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                    footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                    foot_target_velocity, command, flags, grf, stream);
+}
 int qlb_controller_update_host(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
                                const double* base_twist, const double* target_pose, const double* target_twist,
                                const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
                                const uint8_t* contact_mask, const double* phase, const double* mu,
                                const double* normals_world, const double* foot_target_position,
                                const double* foot_target_velocity, double* command, uint32_t* flags, double* grf) {
-  if (!c) return QLB_ERR_NOT_INITIALISED;
-  QLB_GUARD(c->ctx);
-  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;
-  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
-      !phase || !command || !flags)
-    return QLB_ERR_INVALID_ARGUMENT;
-  qlb_context* ctx = c->ctx;
-  DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, c->B);
-  if (rc != QLB_OK) return rc;
-  const size_t B = c->B, cap = ctx->cap;
-  cudaStream_t st = ctx->stream;
-  // inputs: 94 rows in the input staging (kPipe * 54 rows of cap), outputs 24 rows, the three masks one row each
-  constexpr int kIn = 11, kOut = 2;
-  const double* src[kIn] = {q, qd, base_pose, base_twist, target_pose, target_twist, phase, mu, normals_world,
-                            foot_target_position, foot_target_velocity};
-  const int rows[kIn] = {12, 12, 7, 6, 7, 6, 4, 4, 12, 12, 12};
-  static_assert(kPipe * kHostInRows >= 94 && kPipe * kHostOutRows >= 24 && kPipe >= 3, "staging too small for a tick");
-  const uint8_t* msrc[3] = {desired_stance_mask, footstep_mask, contact_mask};
-  double* dst_out[kOut] = {command, grf};
-  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap) {
-    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
-    const double* din[kIn];
-    size_t off = 0;
-    for (int k = 0; k < kIn && rc == QLB_OK; k++) {
-      din[k] = src[k] ? ctx->d_in + off : nullptr;
-      if (src[k] && cudaMemcpy2DAsync(ctx->d_in + off, n * sizeof(double), src[k] + b0, B * sizeof(double), n * sizeof(double),
-                                      rows[k], cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-      off += (size_t)rows[k] * cap;
-    }
-    const uint8_t* dmask[3];
-    for (int k = 0; k < 3 && rc == QLB_OK; k++) {
-      dmask[k] = msrc[k] ? ctx->d_mask + (size_t)k * cap : nullptr;
-      if (msrc[k] && cudaMemcpyAsync(ctx->d_mask + (size_t)k * cap, msrc[k] + b0, n, cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-    }
-    if (rc != QLB_OK) break;
-    double* dout[kOut] = {ctx->d_out, ctx->d_out + 12 * cap};
-    rc = controller_tick(c, n, b0, din[0], din[1], din[2], din[3], din[4], din[5], dmask[0], dmask[1], dmask[2], din[6], din[7],
-                         din[8], din[9], din[10], dout[0], ctx->d_flags, dout[1], st);
-    for (int k = 0; k < kOut && rc == QLB_OK; k++)
-      if (dst_out[k] && cudaMemcpy2DAsync(dst_out[k] + b0, B * sizeof(double), dout[k], n * sizeof(double), n * sizeof(double), 12,
-                                          cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-    if (rc == QLB_OK && cudaMemcpyAsync(flags + b0, ctx->d_flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess)
-      rc = QLB_ERR_CUDA;
-  }
-  // also on failure: no copy may still be reading or writing the caller's buffers when the call returns
-  if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
-  if (rc == QLB_ERR_CUDA) return cuda_fail(ctx, cudaGetLastError(), "qlb_controller_update_host");
-  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
-  return rc;
+  return controller_update_host_t<double>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                          footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                          foot_target_velocity, command, flags, grf);
+}
+int qlb_controller_update_f32_host(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
+                                   const float* base_twist, const float* target_pose, const float* target_twist,
+                                   const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
+                                   const uint8_t* contact_mask, const float* phase, const float* mu,
+                                   const float* normals_world, const float* foot_target_position,
+                                   const float* foot_target_velocity, float* command, uint32_t* flags, float* grf) {
+  return controller_update_host_t<float>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                         footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                         foot_target_velocity, command, flags, grf);
 }
 
 int qlb_controller_get_state(const qlb_controller* c, uint8_t* limb_state, double* efforts, void* stream) {

@@ -261,15 +261,17 @@ __global__ void __launch_bounds__(256) qlb_stats_kernel(unsigned long long B, co
 // (The reference advances its limb index only at the end of the loop body, so a `continue` makes the next foot
 // overwrite the same limb; the per-limb rules below are the evident intent.)
 // One robot i: phase has row pitch ld_phase, limb_state row pitch ld_limb (the controller tick keeps its limb states
-// in arrays of its own batch size).  Returns the stance mask.
+// in arrays of its own batch size).  Returns the stance mask.  A float phase is widened before the comparisons, so the
+// states are those of the double phase of the same value (against float literals, 0.1f > 0.1 would differ).
+template <typename P>
 __device__ __forceinline__ unsigned contact_fsm_robot(unsigned long long i, unsigned des, unsigned fs, unsigned con,
-                                                      const double* __restrict__ phase, unsigned long long ld_phase,
+                                                      const P* __restrict__ phase, unsigned long long ld_phase,
                                                       uint8_t* __restrict__ limb_state, unsigned long long ld_limb) {
   unsigned mask = 0u;
 #pragma unroll
   for (int k = 0; k < 4; k++) {
     const bool d = (des >> k) & 1u, f = (fs >> k) & 1u, c = (con >> k) & 1u;
-    const double ph = phase[(size_t)k * ld_phase + i];
+    const double ph = (double)phase[(size_t)k * ld_phase + i];
     unsigned st = limb_state[(size_t)k * ld_limb + i];
     if (!d) {
       st = QLB_LIMB_SWING_NORMAL;

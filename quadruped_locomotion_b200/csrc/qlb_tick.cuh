@@ -10,6 +10,11 @@
 //
 // Arrays of the caller have row pitch n (the robots of this call); arrays the controller owns have row pitch ld (its
 // batch size) and are passed already offset to the first robot of the call.
+//
+// T is the type of the caller's arrays: double (qlb_controller_update) or float (qlb_controller_update_f32).  The state
+// the controller owns is double either way: a float qd sample goes into the ring exactly, the solve's float torques
+// and the float swing-leg torques are widened into the efforts, and the command is the clamp of the efforts in double,
+// rounded to T.  So the two entry points act on one controller and may be mixed from tick to tick.
 #pragma once
 
 #include "qlb.h"
@@ -20,7 +25,8 @@ namespace qlb {
 
 constexpr int kTickRing = 11;   // joint-velocity samples per robot: the newest and the one 10 periods older
 
-struct TickArgs {
+template <typename T>
+struct TickArgsT {
   unsigned long long n;    // robots in this call = row pitch of the caller's arrays
   unsigned long long ld;   // row pitch of the controller's arrays
   int head;                // ring slot of this tick's sample; the oldest sample is in slot (head + 1) % kTickRing
@@ -28,22 +34,23 @@ struct TickArgs {
   const uint8_t* desired;
   const uint8_t* footstep;   // may be null: every leg supervised
   const uint8_t* contact;
-  const double* phase;       // [4][n]
-  const double* qd;          // [12][n]
+  const T* phase;            // [4][n]
+  const T* qd;               // [12][n]
   uint8_t* limb;             // [4][ld]
   uint8_t* refill;           // [ld]: 1 = fill every ring slot with the next sample
   double* ring;              // [kTickRing][12][ld]
   uint8_t* stance;           // [n] out of the prologue, in of the solve and the epilogue
   // epilogue
   const uint32_t* flags;     // [n] of the solve
-  const double* tau;         // [12][n] of the solve
+  const T* tau;              // [12][n] of the solve
   double* efforts;           // [12][ld]
-  double* command;           // [12][n]
+  T* command;                // [12][n]
   double limit;
-  SwingArgs swing;           // B = n, q, qd, qd_front = oldest ring slot with ld_front = ld, targets, gains
+  SwingArgsT<T> swing;       // B = n, q, qd, qd_front = oldest ring slot with ld_front = ld, targets, gains
 };
 
-__global__ void __launch_bounds__(256) qlb_tick_prologue_kernel(const TickArgs a) {
+template <typename T>
+__global__ void __launch_bounds__(256) qlb_tick_prologue_kernel(const TickArgsT<T> a) {
   const unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long n = a.n, ld = a.ld;
   if (i >= n) return;
@@ -55,12 +62,13 @@ __global__ void __launch_bounds__(256) qlb_tick_prologue_kernel(const TickArgs a
   for (int s = s0; s < s1; s++) {
     double* slot = a.ring + (size_t)s * 12 * ld + i;
 #pragma unroll
-    for (int c = 0; c < 12; c++) slot[(size_t)c * ld] = a.qd[(size_t)c * n + i];
+    for (int c = 0; c < 12; c++) slot[(size_t)c * ld] = (double)a.qd[(size_t)c * n + i];
   }
   if (refill) a.refill[i] = 0;
 }
 
-__global__ void __launch_bounds__(128) qlb_tick_epilogue_kernel(const TickArgs a) {
+template <typename T>
+__global__ void __launch_bounds__(128) qlb_tick_epilogue_kernel(const TickArgsT<T> a) {
   const unsigned long long t = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long n = a.n, ld = a.ld;
   if (t >= 4ull * n) return;
@@ -73,20 +81,20 @@ __global__ void __launch_bounds__(128) qlb_tick_epilogue_kernel(const TickArgs a
     const unsigned status = (a.flags[i] & QLB_FLAG_STATUS_MASK) >> QLB_FLAG_STATUS_SHIFT;
     if (status == QLB_STATE_OK || status == QLB_STATE_NO_STANCE) {
 #pragma unroll
-      for (int j = 0; j < 3; j++) e[j] = a.tau[(size_t)(3 * leg + j) * n + i];
+      for (int j = 0; j < 3; j++) e[j] = (double)a.tau[(size_t)(3 * leg + j) * n + i];
     }
   } else {
-    double tq[3];
+    T tq[3];
     swing_leg_torque(a.swing, leg, i, tq);
     if (isfinite(tq[0]) && isfinite(tq[1]) && isfinite(tq[2])) {
 #pragma unroll
-      for (int j = 0; j < 3; j++) e[j] = tq[j];
+      for (int j = 0; j < 3; j++) e[j] = (double)tq[j];
     }
   }
 #pragma unroll
   for (int j = 0; j < 3; j++) {
     a.efforts[(size_t)(3 * leg + j) * ld + i] = e[j];
-    a.command[(size_t)(3 * leg + j) * n + i] = fmin(fmax(e[j], -a.limit), a.limit);
+    a.command[(size_t)(3 * leg + j) * n + i] = (T)fmin(fmax(e[j], -a.limit), a.limit);
   }
 }
 

@@ -2,7 +2,10 @@
 """Throughput of the controller tick (qlb_controller_update): robot-ticks per second for B robots, device-resident, timed
 with CUDA events after warm-up; per-kernel times from a separate torch.profiler run; the latency of a one-robot tick
 through the host entry point.  Writes one JSON line per configuration (default profiles/tick_bench.jsonl), each with the
-GPU name and power limit read in the same run.
+GPU name and power limit read in the same run.  --dtypes float64,float32 adds the same rows for the FP32 twins
+(qlb_controller_update_f32[_host]) on the same trot rounded to float32.  Every row names its "dtype", the tick kernels
+carry their template argument in the per-kernel times (qlb_tick_epilogue_kernel<double> / <float>), and profiler traces
+are named tick_B{B}_{dtype}.pt.trace.json, also with the default --dtypes float64.
 
 Workload: a trot (LF+RH and RF+LH alternate every 8 ticks, robots spread over the 8 phases) with C3-like joint angles and
 attitudes, base position / twist noise 0.05, targets 4 mm away, swing gains (300, 250, 400) / (10, 12, 8); 8 input sets
@@ -79,12 +82,20 @@ def params():
     return p
 
 
-def bench_device(s, B, ticks, warmup, info, prof_dir):
+def cast(d, dtype):
+    """The floating-point arrays of an input set in `dtype` (masks unchanged)."""
+    return {k: (v.to(dtype).contiguous() if v.is_floating_point() else v) for k, v in d.items()}
+
+
+ENTRY = {torch.float64: "qlb_controller_update", torch.float32: "qlb_controller_update_f32"}
+
+
+def bench_device(s, B, ticks, warmup, info, prof_dir, dtype=torch.float64):
     dev = torch.device("cuda:0")
     g = torch.Generator(device=dev); g.manual_seed(1234)
-    sets = [make_inputs(B, k, dev, g) for k in range(NSETS)]
-    out = dict(command=torch.empty((12, B), dtype=torch.float64, device=dev), flags=torch.empty(B, dtype=torch.int32, device=dev),
-               grf=torch.empty((12, B), dtype=torch.float64, device=dev))
+    sets = [cast(make_inputs(B, k, dev, g), dtype) for k in range(NSETS)]
+    out = dict(command=torch.empty((12, B), dtype=dtype, device=dev), flags=torch.empty(B, dtype=torch.int32, device=dev),
+               grf=torch.empty((12, B), dtype=dtype, device=dev))
     ctrl = capi.Controller(s, B, params())
     stream = torch.cuda.current_stream().cuda_stream
     for k in range(warmup):
@@ -130,21 +141,22 @@ def bench_device(s, B, ticks, warmup, info, prof_dir):
             kernels[name] = kernels.get(name, 0.0) + t / nprof   # us per tick
     if prof_dir:
         os.makedirs(prof_dir, exist_ok=True)
-        prof.export_chrome_trace(os.path.join(prof_dir, f"tick_B{B}.pt.trace.json"))
+        prof.export_chrome_trace(os.path.join(prof_dir, f"tick_B{B}_{str(dtype)[6:]}.pt.trace.json"))
     fl = out["flags"].cpu().numpy().view(np.uint32)
     ctrl.close()
-    return dict(info, entry="qlb_controller_update", robots=B, ticks=ticks, warmup=warmup, ms_per_tick=ms,
+    return dict(info, entry=ENTRY[dtype], dtype=str(dtype)[6:], robots=B, ticks=ticks, warmup=warmup, ms_per_tick=ms,
                 robot_ticks_per_s=B / ms * 1e3, launches_per_tick=launches, solve_state_ms_same_inputs=ms_solve,
                 tick_minus_solve_ms=ms - ms_solve, kernels_us_per_tick=dict(sorted(kernels.items(), key=lambda kv: -kv[1])),
                 ok_fraction_last_tick=float(((fl >> 24) & 7 == 0).mean()))
 
 
-def bench_host(s, ticks, warmup, info):
+def bench_host(s, ticks, warmup, info, dtype=torch.float64):
     dev = torch.device("cuda:0")
     g = torch.Generator(device=dev); g.manual_seed(99)
-    sets = [{k: v.cpu().numpy() for k, v in make_inputs(1, k, dev, g).items()} for k in range(NSETS)]
+    sets = [{k: v.cpu().numpy() for k, v in cast(make_inputs(1, k, dev, g), dtype).items()} for k in range(NSETS)]
     ctrl = capi.Controller(s, 1, params())
-    cmd = np.zeros((12, 1)); fl = np.zeros(1, np.uint32); grf = np.zeros((12, 1))
+    npt = np.float32 if dtype == torch.float32 else np.float64
+    cmd = np.zeros((12, 1), npt); fl = np.zeros(1, np.uint32); grf = np.zeros((12, 1), npt)
     lat = []
     for k in range(warmup + ticks):
         d = sets[k % NSETS]
@@ -155,7 +167,7 @@ def bench_host(s, ticks, warmup, info):
             lat.append((time.perf_counter() - t0) * 1e6)
     ctrl.close()
     lat = np.array(lat)
-    return dict(info, entry="qlb_controller_update_host", robots=1, ticks=ticks, warmup=warmup, us_median=float(np.median(lat)),
+    return dict(info, entry=ENTRY[dtype] + "_host", dtype=str(dtype)[6:], robots=1, ticks=ticks, warmup=warmup, us_median=float(np.median(lat)),
                 us_p99=float(np.percentile(lat, 99)), us_max=float(lat.max()), timer="host clock around the call (it synchronises)")
 
 
@@ -167,14 +179,16 @@ def main():
     ap.add_argument("--host-ticks", type=int, default=2000)
     ap.add_argument("--sizes", default="14,20", help="log2 of the robot counts")
     ap.add_argument("--trace-dir", default=None, help="also write the profiler traces there")
+    ap.add_argument("--dtypes", default="float64", help="array types of the caller: float64 and/or float32, comma-separated")
     a = ap.parse_args()
+    dtypes = [{"float64": torch.float64, "float32": torch.float32}[t.strip()] for t in a.dtypes.split(",")]
     if not torch.cuda.is_available():
         raise SystemExit("tick_bench needs a CUDA device")
     info = gpu_info()
     s = capi.Solver("quadruped_model")
     s.set_limb_dynamics("quadruped_model")
-    rows = [bench_device(s, 1 << int(e), a.ticks, a.warmup, info, a.trace_dir) for e in a.sizes.split(",")]
-    rows.append(bench_host(s, a.host_ticks, 100, info))
+    rows = [bench_device(s, 1 << int(e), a.ticks, a.warmup, info, a.trace_dir, dt) for e in a.sizes.split(",") for dt in dtypes]
+    rows += [bench_host(s, a.host_ticks, 100, info, dt) for dt in dtypes]
     s.close()
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, "w") as f:
