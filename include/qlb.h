@@ -189,7 +189,8 @@ int qlb_solve_wrench(qlb_context* ctx, size_t B, const double* q, const double* 
                      double* netwrench, void* stream);
 
 /* Same, HOST pointers: copies in, solves, copies out, synchronises.  This is what a batch-of-1
- * controller tick calls. */
+ * controller tick calls.  Every *_host entry point synchronises all the streams it used before it returns, on
+ * failure too, so no copy still reads or writes the caller's arrays. */
 int qlb_solve_wrench_host(qlb_context* ctx, size_t B, const double* q, const double* quat_wxyz,
                           const double* wrench, const uint8_t* stance_mask, const double* mu,
                           const double* normals_world, double* grf, double* tau, uint32_t* flags,
@@ -540,7 +541,8 @@ typedef struct qlb_result_record {
 } qlb_result_record;      /* 248 bytes */
 
 /* DEVICE pointers, asynchronous on `stream`: unpack -> qlb_solve_wrench -> pack, in chunks that reuse the
- * context's staging buffers.  Surface normals are the default (0, 0, 1). */
+ * context's staging buffers.  Surface normals are the default (0, 0, 1).  The staging is shared with the other calls
+ * of the context: a later call, on any stream, does not write it before this one has finished with it. */
 int qlb_solve_records(qlb_context* ctx, size_t B, const qlb_wrench_record* records, qlb_result_record* results,
                       void* stream);
 /* HOST pointers (pinned memory recommended): chunks flow through the context's copy / compute pipeline with one

@@ -30,11 +30,24 @@ using namespace qlb;
 #endif
 constexpr int kPipe = QLB_PIPE;   // host entry points: chunks in flight (H2D / kernel / D2H overlap)
 
+// Device memory of a context that only grows (reserve)
+struct DeviceBuffer {
+  unsigned char* p = nullptr;
+  size_t bytes = 0;
+};
+
+// CTAs per SM of the solve kernels of one (interface, core) type pair, [MODE]: the three-pass kernels, and the fused
+// kernel without / with TMA staging (FP64 core only)
+struct SolveOccupancy {
+  int first[2] = {0, 0};
+  int quad[2] = {0, 0};
+  int single[2][2] = {};
+};
+
 struct qlb_context {
   int device = 0;
   int sm_count = 0;
-  int blocks_per_sm_quad[2] = {0, 0};
-  int blocks_per_sm_first[2] = {0, 0};
+  SolveOccupancy occ[3];   // [occ_index<T, C>]: double/double, float/double, float/float
   qlb_params params;
   qlb_leg_model legs[QLB_NUM_LEGS];
   DeviceModel* d_model = nullptr;
@@ -44,37 +57,26 @@ struct qlb_context {
   bool have_limb = false;
   DeviceModelT<float>* d_model_f = nullptr;    // FP32 copies for the _f32 entry points
   DeviceParamsT<float>* d_params_f = nullptr;
-  int blocks_per_sm_quad_f[2] = {0, 0};
-  int blocks_per_sm_first_f[2] = {0, 0};
-  int blocks_per_sm_quad_m[2] = {0, 0};   // FP32 interface + FP64 solver core
-  int blocks_per_sm_first_m[2] = {0, 0};
   int pipeline = QLB_PIPELINE_FUSED;   // qlb_set_pipeline
-  int blocks_per_sm_single[2][2][2] = {};   // [interface type: 0 double, 1 float][MODE][TMA]
   std::recursive_mutex mu;                  // calls on one context from several host threads are serialised (QLB_GUARD)
   int fused_bps_cap = 0;                    // experiments (env QLB_FUSED_BPS): fewer CTAs of the fused kernel per SM
-  bool use_tma = true;    // fused pipeline: stage the inputs with the TMA unit when the arrays allow it
   bool f32_pure = false;  // qlb_set_f32_core: FP32 solver core with in-kernel FP64 rescue, or FP64 core for every state
   unsigned long long* d_counter = nullptr;
-  unsigned* d_list[8] = {};   // second-pass index lists, one per launch slot
-  size_t list_cap[8] = {};
+  DeviceBuffer lists;         // second-pass index lists: 8 launch slots x 3 lists of list_cap entries
+  size_t list_cap = 0;
   uint64_t solve_calls = 0;   // picks the launch slot (counters + list): concurrent launches never share one
   cudaEvent_t slot_done[8] = {};  // recorded after the last pass of the call that used the slot; the next user waits on it
   int last_slot = 0;
   double* d_stats = nullptr;
   cudaStream_t stream = nullptr;  // used by the *_host entry points
   cudaStream_t pipe[kPipe] = {};  // chunk pipeline of the *_host entry points
-  // device staging for the *_host entry points
-  double* d_in = nullptr;
-  double* d_out = nullptr;
-  uint8_t* d_mask = nullptr;
-  uint32_t* d_flags = nullptr;
-  unsigned char* d_prev = nullptr;  // staging of qlb_preview_plan_host
-  size_t prev_cap = 0;
-  unsigned char* d_qp = nullptr;    // staging of qlb_qp_dense_host
-  size_t qp_bytes = 0;
-  unsigned char* d_rec = nullptr;   // record staging of qlb_solve_records_host: kPipe x cap x (216 + 248) bytes
-  size_t rec_cap = 0;
+  // staging of the host entry points and qlb_solve_records
+  DeviceBuffer soa;    // SoA rows of kPipe slots of `cap` states (soa_slot)
   size_t cap = 0;
+  cudaEvent_t soa_free = nullptr;   // recorded after the last asynchronous use of `soa` (qlb_solve_records)
+  DeviceBuffer rec;    // records of qlb_solve_records_host: kPipe x cap x (216 + 248) bytes
+  DeviceBuffer prev;   // qlb_preview_plan_host
+  DeviceBuffer qp;     // qlb_qp_dense_host
   uint64_t launches = 0;
   char last_error[256] = {0};
 };
@@ -117,6 +119,41 @@ int cuda_fail(qlb_context* ctx, cudaError_t e, const char* what) {
     cudaError_t e__ = (call);                                 \
     if (e__ != cudaSuccess) return cuda_fail(ctx, e__, #call); \
   } while (0)
+
+#define QLB_TRY(call)                        \
+  do {                                       \
+    const int rc__ = (call);                 \
+    if (rc__ != QLB_OK) return rc__;         \
+  } while (0)
+
+// The one rule of every staging buffer: the device is synchronised before the old buffer is freed (work on any stream
+// may still use it); when the allocation fails the buffer is left empty.
+int reserve(qlb_context* ctx, DeviceBuffer& b, size_t bytes) {
+  if (bytes <= b.bytes) return QLB_OK;
+  QLB_CUDA(ctx, cudaDeviceSynchronize());
+  cudaFree(b.p);
+  b.p = nullptr;
+  b.bytes = 0;
+  if (cudaMalloc(&b.p, bytes) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
+  b.bytes = bytes;
+  return QLB_OK;
+}
+
+size_t pow2_at_least(size_t n, size_t lo) {
+  while (lo < n) lo *= 2;
+  return lo;
+}
+
+// One thread per item: ceil(items / threads) blocks of `threads`.
+template <typename... P, typename... A>
+int launch_items(qlb_context* ctx, unsigned long long items, unsigned threads, cudaStream_t st, void (*kernel)(P...), A... args) {
+  const unsigned long long blocks = (items + threads - 1) / threads;
+  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
+  kernel<<<(unsigned)blocks, threads, 0, st>>>(args...);
+  QLB_CUDA(ctx, cudaGetLastError());
+  ctx->launches++;
+  return QLB_OK;
+}
 
 // URDF <origin rpy> -> rotation matrix, through the quaternion like urdfdom + KDL do.
 void rpy_to_rot(const double rpy[3], double R[9]) {
@@ -233,35 +270,33 @@ int prepare_slot(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st) {
   a.list_count = reinterpret_cast<unsigned*>(a.counter + 3);
   a.list2_count = reinterpret_cast<unsigned*>(a.counter + 4);
   QLB_CUDA(ctx, cudaMemsetAsync(a.counter, 0, 8 * sizeof(unsigned long long), st));
-  if (ctx->list_cap[slot] < a.B) {  // grow the index lists of all slots at once (rare; synchronises)
-    QLB_CUDA(ctx, cudaDeviceSynchronize());
-    size_t cap = 1024;
-    while (cap < a.B) cap *= 2;
-    for (int i = 0; i < 8; i++) {
-      if (ctx->list_cap[i] >= cap) continue;
-      cudaFree(ctx->d_list[i]);
-      ctx->d_list[i] = nullptr;
-      ctx->list_cap[i] = 0;
-      if (cudaMalloc(&ctx->d_list[i], 3 * cap * sizeof(unsigned)) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
-      ctx->list_cap[i] = cap;
-    }
+  if (ctx->list_cap < a.B) {  // grow the index lists of all slots at once (rare; synchronises)
+    const size_t cap = pow2_at_least(a.B, 1024);
+    ctx->list_cap = 0;
+    QLB_TRY(reserve(ctx, ctx->lists, 8 * 3 * cap * sizeof(unsigned)));
+    ctx->list_cap = cap;
   }
-  a.list = ctx->d_list[slot];
-  a.list2 = ctx->d_list[slot] + ctx->list_cap[slot];
-  a.list_pat = ctx->d_list[slot] + 2 * ctx->list_cap[slot];
+  unsigned* list = reinterpret_cast<unsigned*>(ctx->lists.p) + (size_t)slot * 3 * ctx->list_cap;
+  a.list = list;
+  a.list2 = list + ctx->list_cap;
+  a.list_pat = list + 2 * ctx->list_cap;
   return QLB_OK;
 }
+
+template <typename T, typename C>
+constexpr int occ_index() { return sizeof(T) == 8 ? 0 : sizeof(C) == 8 ? 1 : 2; }
 
 // The three passes of the leg-per-lane kernels.  pass 1: everything up to the unconstrained minimiser;
 // pass 2: active-set rounds on what is left; pass 3: interior point on what is still left.  The later
 // grids are sized for the worst case and read the list lengths on the device (no host synchronisation
 // between the passes).
 template <typename T, typename C, int MODE>
-int launch_quad(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st, const int bps_first, const int bps_quad) {
+int launch_quad(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st) {
+  const SolveOccupancy& occ = ctx->occ[occ_index<T, C>()];
   const unsigned long long nb8 = (a.B + 7) / 8;
   const unsigned long long wantq = (nb8 + (kQuadThreads / 32) - 1) / (kQuadThreads / 32);
-  const unsigned long long capq = (unsigned long long)ctx->sm_count * bps_quad;
-  const unsigned long long capf = (unsigned long long)ctx->sm_count * bps_first;
+  const unsigned long long capq = (unsigned long long)ctx->sm_count * occ.quad[MODE];
+  const unsigned long long capf = (unsigned long long)ctx->sm_count * occ.first[MODE];
   const unsigned gq = (unsigned)(wantq < capq ? wantq : capq);
   qlb_quad_first_kernel<T, C, MODE><<<(unsigned)(wantq < capf ? wantq : capf), kQuadThreads, 0, st>>>(a);
   QLB_CUDA(ctx, cudaGetLastError());
@@ -323,12 +358,13 @@ bool make_mask_map(CUtensorMap* m, const uint8_t* ptr, unsigned long long B, int
 // the fused kernel (qlb_solve_single.cuh) + the interior-point kernel for the states its rounds could not verify
 // (normally none: it finds an empty list and returns)
 template <typename T, typename C, int MODE>
-int launch_single(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st, const int bps_ipm) {
+int launch_single(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st) {
+  const SolveOccupancy& occ = ctx->occ[occ_index<T, C>()];
   using SG = Staging<T, MODE, QLB_SUPER>;
   using FL = FusedLayout<T, C, MODE, QLB_SUPER>;
   const T* src[SG::kNumSeg];
   for (int s = 0; s < SG::kNumSeg; s++) src[s] = SG::source(a, s);
-  bool tma = ctx->use_tma && a.B >= 64 && a.B < 0x7fffff00ull && ((a.B * sizeof(T)) % 16 == 0);
+  bool tma = a.B >= 64 && a.B < 0x7fffff00ull && ((a.B * sizeof(T)) % 16 == 0);
   for (int s = 0; s < SG::kNumSeg && tma; s++)
     if (src[s] && !aligned16(src[s])) tma = false;
   FusedMaps maps;
@@ -338,7 +374,7 @@ int launch_single(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st, const int
   if (tma && (SG::kCols < 16 || !aligned16(a.mask) || !make_mask_map(&maps.mask, a.mask, a.B, SG::kCols))) tma = false;
   const unsigned long long ntiles = (a.B + 7) / 8;
   const unsigned long long want = (ntiles + kFusedWarps - 1) / kFusedWarps;
-  int bps = ctx->blocks_per_sm_single[sizeof(T) == 4 ? 1 : 0][MODE][tma ? 1 : 0];
+  int bps = occ.single[MODE][tma ? 1 : 0];
   if (ctx->fused_bps_cap > 0 && bps > ctx->fused_bps_cap) bps = ctx->fused_bps_cap;
   const unsigned long long cap = (unsigned long long)ctx->sm_count * bps;
   const unsigned grid = (unsigned)(want < cap ? want : cap);
@@ -346,7 +382,7 @@ int launch_single(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st, const int
   else qlb_single_kernel<T, C, MODE, QLB_SUPER, false><<<grid, kFusedThreads, FL::kTotal, st>>>(a, maps);
   QLB_CUDA(ctx, cudaGetLastError());
   ctx->launches++;
-  const unsigned long long capq = (unsigned long long)ctx->sm_count * bps_ipm;
+  const unsigned long long capq = (unsigned long long)ctx->sm_count * occ.quad[MODE];
   const unsigned long long wantq = (ntiles + 3) / 4;
   qlb_quad_kernel<T, C, MODE, 2><<<(unsigned)(wantq < capq ? wantq : capq), kQuadThreads, 0, st>>>(a);
   QLB_CUDA(ctx, cudaGetLastError());
@@ -355,10 +391,24 @@ int launch_single(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st, const int
   return QLB_OK;
 }
 
-template <typename T, typename C, int MODE>
+// ctx->occ of one type pair: the three-pass kernels of both modes
+template <typename T, typename C>
+bool query_occupancy(qlb_context* ctx) {
+  SolveOccupancy& o = ctx->occ[occ_index<T, C>()];
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.quad[0], qlb_quad_kernel<T, C, 0, 2>, kQuadThreads, 0) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.quad[1], qlb_quad_kernel<T, C, 1, 2>, kQuadThreads, 0) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.first[0], qlb_quad_first_kernel<T, C, 0>, kQuadThreads, 0) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o.first[1], qlb_quad_first_kernel<T, C, 1>, kQuadThreads, 0) != cudaSuccess)
+    return false;
+  return o.quad[0] >= 1 && o.quad[1] >= 1 && o.first[0] >= 1 && o.first[1] >= 1;
+}
+
+// ctx->occ.single of the fused kernel (FP64 core) for one interface type and mode
+template <typename T, int MODE>
 bool prepare_single_kernels(qlb_context* ctx) {
+  using C = double;
   using FL = FusedLayout<T, C, MODE, QLB_SUPER>;
-  int* out = ctx->blocks_per_sm_single[sizeof(T) == 4 ? 1 : 0][MODE];
+  int* out = ctx->occ[occ_index<T, C>()].single[MODE];
   if (cudaFuncSetAttribute(qlb_single_kernel<T, C, MODE, QLB_SUPER, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL::kTotal) != cudaSuccess ||
       cudaFuncSetAttribute(qlb_single_kernel<T, C, MODE, QLB_SUPER, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FL::kTotal) != cudaSuccess ||
       cudaFuncSetAttribute(qlb_single_kernel<T, C, MODE, QLB_SUPER, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) != cudaSuccess ||
@@ -370,40 +420,83 @@ bool prepare_single_kernels(qlb_context* ctx) {
   return out[0] >= 1 && out[1] >= 1;
 }
 
-template <int MODE>
-int launch_solve(qlb_context* ctx, SolveArgs& a, cudaStream_t st) {
-  const int rc = prepare_slot(ctx, a, st);
-  if (rc != QLB_OK) return rc;
-  if (ctx->pipeline == QLB_PIPELINE_FUSED) return launch_single<double, double, MODE>(ctx, a, st, ctx->blocks_per_sm_quad[MODE]);
-  return launch_quad<double, double, MODE>(ctx, a, st, ctx->blocks_per_sm_first[MODE], ctx->blocks_per_sm_quad[MODE]);
+// The FP64 interface runs the FP64 core; the FP32 interface the FP64 core or, with qlb_set_f32_core, the FP32 core
+// (three-pass pipeline only).
+template <typename T, int MODE>
+int launch_solve(qlb_context* ctx, SolveArgsT<T>& a, cudaStream_t st) {
+  QLB_TRY(prepare_slot(ctx, a, st));
+  if constexpr (sizeof(T) == 4) {
+    if (ctx->f32_pure) return launch_quad<float, float, MODE>(ctx, a, st);
+  }
+  if (ctx->pipeline == QLB_PIPELINE_FUSED) return launch_single<T, double, MODE>(ctx, a, st);
+  return launch_quad<T, double, MODE>(ctx, a, st);
 }
 
-// FP32 twins: FP32 interface with the FP64 or the FP32 solver core (qlb_set_f32_core)
-template <int MODE>
-int launch_solve_f32(qlb_context* ctx, SolveArgsT<float>& a, cudaStream_t st) {
-  const int rc = prepare_slot(ctx, a, st);
-  if (rc != QLB_OK) return rc;
-  if (ctx->f32_pure) return launch_quad<float, float, MODE>(ctx, a, st, ctx->blocks_per_sm_first_f[MODE], ctx->blocks_per_sm_quad_f[MODE]);
-  if (ctx->pipeline == QLB_PIPELINE_FUSED) return launch_single<float, double, MODE>(ctx, a, st, ctx->blocks_per_sm_quad_m[MODE]);
-  return launch_quad<float, double, MODE>(ctx, a, st, ctx->blocks_per_sm_first_m[MODE], ctx->blocks_per_sm_quad_m[MODE]);
+// SoA staging of the host entry points and qlb_solve_records: kPipe slots of `cap` states, laid out as
+// [kPipe][kHostInRows][cap] and [kPipe][kHostOutRows][cap] doubles, [kPipe][cap] flags and [kPipe][cap] mask bytes.
+// cap is a power of two >= 1024: cap % 16 == 0 keeps every row block 16-byte aligned, so that launch_single's choice of
+// TMA does not depend on the chunk.
+constexpr size_t kSoaBytesPerState = (kHostInRows + kHostOutRows) * sizeof(double) + sizeof(uint32_t) + 1;
+struct SoaSlot {
+  double* in;
+  double* out;
+  uint32_t* flags;
+  uint8_t* mask;
+};
+SoaSlot soa_slot(const qlb_context* ctx, int slot) {
+  const size_t cap = ctx->cap;
+  double* in = reinterpret_cast<double*>(ctx->soa.p);
+  double* out = in + kPipe * cap * kHostInRows;
+  uint32_t* flags = reinterpret_cast<uint32_t*>(out + kPipe * cap * kHostOutRows);
+  uint8_t* mask = reinterpret_cast<uint8_t*>(flags + kPipe * cap);
+  return {in + slot * cap * kHostInRows, out + slot * cap * kHostOutRows, flags + slot * cap, mask + slot * cap};
 }
 
-// staging of the host entry points: kPipe slots of `cap` states each (cap <= kChunk)
-int ensure_capacity(qlb_context* ctx, size_t B) {
+int reserve_soa(qlb_context* ctx, size_t B) {
   if (B > kChunk) B = kChunk;
   if (B <= ctx->cap) return QLB_OK;
-  size_t cap = ctx->cap ? ctx->cap : 1024;
-  while (cap < B) cap *= 2;
-  cap = (cap + 15) & ~size_t(15);
-  cudaFree(ctx->d_in); cudaFree(ctx->d_out); cudaFree(ctx->d_mask); cudaFree(ctx->d_flags);
-  ctx->d_in = ctx->d_out = nullptr; ctx->d_mask = nullptr; ctx->d_flags = nullptr; ctx->cap = 0;
-  if (cudaMalloc(&ctx->d_in, kPipe * cap * kHostInRows * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&ctx->d_out, kPipe * cap * kHostOutRows * sizeof(double)) != cudaSuccess ||
-      cudaMalloc(&ctx->d_mask, kPipe * cap) != cudaSuccess || cudaMalloc(&ctx->d_flags, kPipe * cap * sizeof(uint32_t)) != cudaSuccess) {
-    cudaGetLastError();
-    return QLB_ERR_ALLOC;
-  }
+  const size_t cap = pow2_at_least(B, ctx->cap ? ctx->cap : 1024);
+  ctx->cap = 0;
+  QLB_TRY(reserve(ctx, ctx->soa, kPipe * cap * kSoaBytesPerState));
   ctx->cap = cap;
+  return QLB_OK;
+}
+
+// Runs body(b0, n, slot, stream) over [0, B) in chunks of `chunk` states: chunk i on pipeline stream i % kPipe with
+// staging slot i % kPipe, or all of them on the context stream with slot 0.  Each stream waits for the last
+// asynchronous user of the SoA staging before its first chunk.  Every stream it enqueued on is synchronised before it
+// returns, on failure too: no copy may still be reading or writing the caller's buffers.
+template <typename F>
+int for_chunks(qlb_context* ctx, size_t B, size_t chunk, bool pipelined, F&& body) {
+  cudaStream_t* streams = pipelined ? ctx->pipe : &ctx->stream;
+  const int nstreams = pipelined ? kPipe : 1;
+  int used = 0, rc = QLB_OK;
+  for (size_t b0 = 0, i = 0; b0 < B && rc == QLB_OK; b0 += chunk, i++) {
+    const int slot = (int)(i % nstreams);
+    if (used <= slot) {
+      used = slot + 1;
+      const cudaError_t e = cudaStreamWaitEvent(streams[slot], ctx->soa_free, 0);
+      if (e != cudaSuccess) { rc = cuda_fail(ctx, e, "cudaStreamWaitEvent"); break; }
+    }
+    rc = body(b0, B - b0 < chunk ? B - b0 : chunk, slot, streams[slot]);
+  }
+  for (int i = 0; i < used; i++) {
+    const cudaError_t e = cudaStreamSynchronize(streams[i]);
+    if (e != cudaSuccess && rc == QLB_OK) rc = cuda_fail(ctx, e, "cudaStreamSynchronize");
+  }
+  return rc;
+}
+
+// Rows [0, rows) of columns [b0, b0 + n) of a host array with row pitch B, to or from a device block with row pitch n.
+// A null host array is skipped.
+template <typename T>
+int rows_to_device(qlb_context* ctx, T* d, const T* h, size_t rows, size_t b0, size_t n, size_t B, cudaStream_t st) {
+  if (h) QLB_CUDA(ctx, cudaMemcpy2DAsync(d, n * sizeof(T), h + b0, B * sizeof(T), n * sizeof(T), rows, cudaMemcpyHostToDevice, st));
+  return QLB_OK;
+}
+template <typename T>
+int rows_to_host(qlb_context* ctx, T* h, const T* d, size_t rows, size_t b0, size_t n, size_t B, cudaStream_t st) {
+  if (h) QLB_CUDA(ctx, cudaMemcpy2DAsync(h + b0, B * sizeof(T), d, n * sizeof(T), n * sizeof(T), rows, cudaMemcpyDeviceToHost, st));
   return QLB_OK;
 }
 
@@ -484,50 +577,45 @@ const ParamKey kParamKeys[] = {
     {"/balance_controller/virtual_model_controller/yaw/kd", 8, 2}, {"/balance_controller/virtual_model_controller/yaw/kff", 9, 2},
 };
 constexpr int kNumParamKeys = (int)(sizeof(kParamKeys) / sizeof(kParamKeys[0]));
+
+// index of a key in kParamKeys, or -1
+int find_param_key(const char* key) {
+  for (int k = 0; k < kNumParamKeys; k++)
+    if (std::strcmp(key, kParamKeys[k].path) == 0) return k;
+  return -1;
+}
+
+double* param_field(qlb_params* p, int k) {
+  const int i = kParamKeys[k].index;
+  switch (kParamKeys[k].group) {
+    case 0: return &p->wrench_weights[i];
+    case 1: return &p->ground_force_weight;
+    case 2: return &p->friction_default;
+    case 3: return &p->min_normal_force;
+    case 4: return &p->kp_translation[i];
+    case 5: return &p->kd_translation[i];
+    case 6: return &p->kff_translation[i];
+    case 7: return &p->kp_rotation[i];
+    case 8: return &p->kd_rotation[i];
+    default: return &p->kff_rotation[i];
+  }
+}
 }  // namespace
 
 int qlb_params_set_key(qlb_params* p, const char* key, double value) {
   if (!p || !key) return QLB_ERR_INVALID_ARGUMENT;
-  for (int k = 0; k < kNumParamKeys; k++) {
-    if (std::strcmp(key, kParamKeys[k].path) != 0) continue;
-    const int i = kParamKeys[k].index;
-    switch (kParamKeys[k].group) {
-      case 0: p->wrench_weights[i] = value; break;
-      case 1: p->ground_force_weight = value; break;
-      case 2: p->friction_default = value; break;
-      case 3: p->min_normal_force = value; break;
-      case 4: p->kp_translation[i] = value; break;
-      case 5: p->kd_translation[i] = value; break;
-      case 6: p->kff_translation[i] = value; break;
-      case 7: p->kp_rotation[i] = value; break;
-      case 8: p->kd_rotation[i] = value; break;
-      default: p->kff_rotation[i] = value; break;
-    }
-    return k;   // index of the key (>= 0)
-  }
-  return QLB_ERR_INVALID_ARGUMENT;
+  const int k = find_param_key(key);
+  if (k < 0) return QLB_ERR_INVALID_ARGUMENT;
+  *param_field(p, k) = value;
+  return k;   // index of the key (>= 0)
 }
 
 int qlb_params_get_key(const qlb_params* p, const char* key, double* value) {
   if (!p || !key || !value) return QLB_ERR_INVALID_ARGUMENT;
-  for (int k = 0; k < kNumParamKeys; k++) {
-    if (std::strcmp(key, kParamKeys[k].path) != 0) continue;
-    const int i = kParamKeys[k].index;
-    switch (kParamKeys[k].group) {
-      case 0: *value = p->wrench_weights[i]; break;
-      case 1: *value = p->ground_force_weight; break;
-      case 2: *value = p->friction_default; break;
-      case 3: *value = p->min_normal_force; break;
-      case 4: *value = p->kp_translation[i]; break;
-      case 5: *value = p->kd_translation[i]; break;
-      case 6: *value = p->kff_translation[i]; break;
-      case 7: *value = p->kp_rotation[i]; break;
-      case 8: *value = p->kd_rotation[i]; break;
-      default: *value = p->kff_rotation[i]; break;
-    }
-    return k;
-  }
-  return QLB_ERR_INVALID_ARGUMENT;
+  const int k = find_param_key(key);
+  if (k < 0) return QLB_ERR_INVALID_ARGUMENT;
+  *value = *param_field(const_cast<qlb_params*>(p), k);
+  return k;
 }
 
 int qlb_params_num_keys(void) { return kNumParamKeys; }
@@ -633,6 +721,7 @@ int qlb_create(qlb_context** out, const qlb_leg_model legs[QLB_NUM_LEGS], const 
     if (cudaStreamCreateWithFlags(&ctx->pipe[i], cudaStreamNonBlocking) != cudaSuccess) return fail(QLB_ERR_CUDA);
   for (int i = 0; i < 8; i++)
     if (cudaEventCreateWithFlags(&ctx->slot_done[i], cudaEventDisableTiming) != cudaSuccess) return fail(QLB_ERR_CUDA);
+  if (cudaEventCreateWithFlags(&ctx->soa_free, cudaEventDisableTiming) != cudaSuccess) return fail(QLB_ERR_CUDA);
   DeviceModel hm;
   build_device_model(legs, &hm);
   if (cudaMemcpy(ctx->d_model, &hm, sizeof hm, cudaMemcpyHostToDevice) != cudaSuccess) return fail(QLB_ERR_CUDA);
@@ -640,35 +729,14 @@ int qlb_create(qlb_context** out, const qlb_leg_model legs[QLB_NUM_LEGS], const 
   narrow_model(hm, &hmf);
   if (cudaMemcpy(ctx->d_model_f, &hmf, sizeof hmf, cudaMemcpyHostToDevice) != cudaSuccess) return fail(QLB_ERR_CUDA);
   if (qlb_set_params(ctx, p) != QLB_OK) return fail(QLB_ERR_CUDA);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad[0], qlb_quad_kernel<double, double, 0, 2>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad[1], qlb_quad_kernel<double, double, 1, 2>, kQuadThreads, 0) != cudaSuccess)
-    return fail(QLB_ERR_CUDA);
-  if (ctx->blocks_per_sm_quad[0] < 1 || ctx->blocks_per_sm_quad[1] < 1) return fail(QLB_ERR_CUDA);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first[0], qlb_quad_first_kernel<double, double, 0>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first[1], qlb_quad_first_kernel<double, double, 1>, kQuadThreads, 0) != cudaSuccess)
-    return fail(QLB_ERR_CUDA);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad_f[0], qlb_quad_kernel<float, float, 0, 2>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad_f[1], qlb_quad_kernel<float, float, 1, 2>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first_f[0], qlb_quad_first_kernel<float, float, 0>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first_f[1], qlb_quad_first_kernel<float, float, 1>, kQuadThreads, 0) != cudaSuccess)
-    return fail(QLB_ERR_CUDA);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad_m[0], qlb_quad_kernel<float, double, 0, 2>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_quad_m[1], qlb_quad_kernel<float, double, 1, 2>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first_m[0], qlb_quad_first_kernel<float, double, 0>, kQuadThreads, 0) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm_first_m[1], qlb_quad_first_kernel<float, double, 1>, kQuadThreads, 0) != cudaSuccess)
-    return fail(QLB_ERR_CUDA);
-  if (!prepare_single_kernels<double, double, 0>(ctx) || !prepare_single_kernels<double, double, 1>(ctx) ||
-      !prepare_single_kernels<float, double, 0>(ctx) || !prepare_single_kernels<float, double, 1>(ctx)) {
+  if (!query_occupancy<double, double>(ctx) || !query_occupancy<float, float>(ctx) || !query_occupancy<float, double>(ctx) ||
+      !prepare_single_kernels<double, 0>(ctx) || !prepare_single_kernels<double, 1>(ctx) ||
+      !prepare_single_kernels<float, 0>(ctx) || !prepare_single_kernels<float, 1>(ctx)) {
     cudaGetLastError();
     return fail(QLB_ERR_CUDA);
   }
   if (const char* e = std::getenv("QLB_FUSED_BPS")) ctx->fused_bps_cap = std::atoi(e);
-  if (const char* e = std::getenv("QLB_PIPELINE")) {   // experiments: three_pass | fused | fused_notma
-    if (!std::strcmp(e, "three_pass")) ctx->pipeline = QLB_PIPELINE_THREE_PASS;
-
-    if (!std::strcmp(e, "fused_notma")) ctx->use_tma = false;
-  }
-  if (max_batch > 0 && ensure_capacity(ctx, max_batch) != QLB_OK) return fail(QLB_ERR_ALLOC);
+  if (max_batch > 0 && reserve_soa(ctx, max_batch) != QLB_OK) return fail(QLB_ERR_ALLOC);
   *out = ctx;
   return QLB_OK;
 }
@@ -681,10 +749,10 @@ int qlb_destroy(qlb_context* ctx) {
     if (ctx->pipe[i]) { cudaStreamSynchronize(ctx->pipe[i]); cudaStreamDestroy(ctx->pipe[i]); }
   cudaFree(ctx->d_model); cudaFree(ctx->d_params); cudaFree(ctx->d_counter); cudaFree(ctx->d_stats);
   cudaFree(ctx->d_model_f); cudaFree(ctx->d_params_f); cudaFree(ctx->d_limb); cudaFree(ctx->d_limb_f);
-  cudaFree(ctx->d_in); cudaFree(ctx->d_out); cudaFree(ctx->d_mask); cudaFree(ctx->d_flags); cudaFree(ctx->d_rec); cudaFree(ctx->d_qp); cudaFree(ctx->d_prev);
-  for (int i = 0; i < 8; i++) cudaFree(ctx->d_list[i]);
+  for (DeviceBuffer* b : {&ctx->lists, &ctx->soa, &ctx->rec, &ctx->prev, &ctx->qp}) cudaFree(b->p);
   for (int i = 0; i < 8; i++)
     if (ctx->slot_done[i]) cudaEventDestroy(ctx->slot_done[i]);
+  if (ctx->soa_free) cudaEventDestroy(ctx->soa_free);
   cudaGetLastError();
   delete ctx;
   return QLB_OK;
@@ -731,7 +799,8 @@ int qlb_set_pipeline(qlb_context* ctx, int pipeline) {
 
 uint64_t qlb_launch_count(const qlb_context* ctx) { return ctx ? ctx->launches : 0; }
 
-// ---- device-pointer entry points (T = double, and float for the _f32 twins)
+// ---- solve entry points (T = double, and float for the _f32 twins).  Each device-pointer / host-pointer twin pair goes
+// through one function that checks the arguments and then launches on `stream` or runs the host pipeline.
 extern "C++" {
 namespace {
 
@@ -740,141 +809,97 @@ template <> struct Typed<double> {
   static const DeviceModel* model(const qlb_context* c) { return c->d_model; }
   static const DeviceLimbDynamics* limb(const qlb_context* c) { return c->d_limb; }
   static const DeviceParams* params(const qlb_context* c) { return c->d_params; }
-  template <int MODE> static int launch(qlb_context* c, SolveArgs& a, cudaStream_t st) { return launch_solve<MODE>(c, a, st); }
 };
 template <> struct Typed<float> {
   static const DeviceModelT<float>* model(const qlb_context* c) { return c->d_model_f; }
   static const DeviceLimbDynamicsT<float>* limb(const qlb_context* c) { return c->d_limb_f; }
   static const DeviceParamsT<float>* params(const qlb_context* c) { return c->d_params_f; }
-  template <int MODE> static int launch(qlb_context* c, SolveArgsT<float>& a, cudaStream_t st) { return launch_solve_f32<MODE>(c, a, st); }
 };
+
+// Host pipeline of the solve: copy in, solve, copy out, synchronise.
+// Large batches are cut into chunks of kChunk states that flow through kPipe streams, so that the H2D
+// copy of chunk i+1, the kernel of chunk i and the D2H copy of chunk i-1 overlap (PCIe is full duplex).
+// The arrays are SoA with row pitch B, so a chunk is a column range: one 2-D copy per array.
+// solve(n, in, mask, out, flags, stream) runs the device-pointer solve on the staged arrays of one chunk.
+template <typename P> struct HostRows { P h; int rows; };   // array (may be null) and its component count
+
+template <typename T, typename F>
+int run_host_pipeline(qlb_context* ctx, size_t B, const HostRows<const T*>* in, int nin, const uint8_t* mask,
+                      const HostRows<T*>* out, int nout, uint32_t* flags, F&& solve) {
+  QLB_TRY(reserve_soa(ctx, B));
+  const size_t cap = ctx->cap;
+  return for_chunks(ctx, B, cap, true, [&](size_t b0, size_t n, int slot, cudaStream_t st) -> int {
+    // the staging is sized for FP64; the FP32 twins use the first half of each slot
+    const SoaSlot s = soa_slot(ctx, slot);
+    T* din = reinterpret_cast<T*>(s.in);
+    T* dout = reinterpret_cast<T*>(s.out);
+    const T* dptr_in[8];
+    T* dptr_out[4];
+    for (int k = 0; k < nin; k++) {
+      dptr_in[k] = in[k].h ? din : nullptr;
+      QLB_TRY(rows_to_device(ctx, din, in[k].h, in[k].rows, b0, n, B, st));
+      din += (size_t)in[k].rows * cap;   // fixed block sizes keep every block 16-byte aligned (cap % 16 == 0)
+    }
+    QLB_CUDA(ctx, cudaMemcpyAsync(s.mask, mask + b0, n, cudaMemcpyHostToDevice, st));
+    for (int k = 0; k < nout; k++) {
+      dptr_out[k] = out[k].h ? dout : nullptr;
+      dout += (size_t)out[k].rows * cap;
+    }
+    QLB_TRY(solve(n, dptr_in, s.mask, dptr_out, s.flags, st));
+    for (int k = 0; k < nout; k++) QLB_TRY(rows_to_host(ctx, out[k].h, dptr_out[k], out[k].rows, b0, n, B, st));
+    QLB_CUDA(ctx, cudaMemcpyAsync(flags + b0, s.flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    return QLB_OK;
+  });
+}
 
 template <typename T>
 int solve_wrench_t(qlb_context* ctx, size_t B, const T* q, const T* quat_wxyz, const T* wrench, const uint8_t* stance_mask,
-                   const T* mu, const T* normals_world, T* grf, T* tau, uint32_t* flags, T* netwrench, void* stream) {
+                   const T* mu, const T* normals_world, T* grf, T* tau, uint32_t* flags, T* netwrench, void* stream, bool host) {
   if (!ctx) return QLB_ERR_NOT_INITIALISED;
   if (B == 0) return QLB_OK;
   if (!q || !quat_wxyz || !wrench || !stance_mask || !grf || !tau || !flags) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
+  if (host) {
+    const HostRows<const T*> in[5] = {{q, 12}, {quat_wxyz, 4}, {wrench, 6}, {mu, 4}, {normals_world, 12}};
+    const HostRows<T*> out[3] = {{grf, 12}, {tau, 12}, {netwrench, 6}};
+    return run_host_pipeline<T>(ctx, B, in, 5, stance_mask, out, 3, flags,
+                                [&](size_t n, const T* const* i, const uint8_t* m, T* const* o, uint32_t* f, cudaStream_t st) {
+                                  return solve_wrench_t<T>(ctx, n, i[0], i[1], i[2], m, i[3], i[4], o[0], o[1], f, o[2], st, false);
+                                });
+  }
   SolveArgsT<T> a;
   std::memset(&a, 0, sizeof a);
   a.B = B; a.q = q; a.quat = quat_wxyz; a.wrench = wrench; a.mask = stance_mask; a.mu = mu; a.normals = normals_world;
   a.grf = grf; a.tau = tau; a.flags = flags; a.netwrench = netwrench;
-  a.counter = ctx->d_counter; a.model = Typed<T>::model(ctx); a.params = Typed<T>::params(ctx); a.params64 = ctx->d_params;
-  return Typed<T>::template launch<0>(ctx, a, static_cast<cudaStream_t>(stream));
+  a.model = Typed<T>::model(ctx); a.params = Typed<T>::params(ctx); a.params64 = ctx->d_params;
+  return launch_solve<T, 0>(ctx, a, static_cast<cudaStream_t>(stream));
 }
 
 template <typename T>
 int solve_state_t(qlb_context* ctx, size_t B, const T* q, const T* base_pose, const T* base_twist, const T* target_pose,
                   const T* target_twist, const uint8_t* stance_mask, const T* mu, const T* normals_world, T* grf, T* tau,
-                  uint32_t* flags, T* netwrench, T* wrench_out, void* stream) {
+                  uint32_t* flags, T* netwrench, T* wrench_out, void* stream, bool host) {
   if (!ctx) return QLB_ERR_NOT_INITIALISED;
   if (B == 0) return QLB_OK;
   if (!q || !base_pose || !base_twist || !target_pose || !target_twist || !stance_mask || !grf || !tau || !flags)
     return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
+  if (host) {
+    const HostRows<const T*> in[7] = {{q, 12}, {base_pose, 7}, {base_twist, 6}, {target_pose, 7}, {target_twist, 6}, {mu, 4}, {normals_world, 12}};
+    const HostRows<T*> out[4] = {{grf, 12}, {tau, 12}, {netwrench, 6}, {wrench_out, 6}};
+    return run_host_pipeline<T>(ctx, B, in, 7, stance_mask, out, 4, flags,
+                                [&](size_t n, const T* const* i, const uint8_t* m, T* const* o, uint32_t* f, cudaStream_t st) {
+                                  return solve_state_t<T>(ctx, n, i[0], i[1], i[2], i[3], i[4], m, i[5], i[6], o[0], o[1], f, o[2],
+                                                          o[3], st, false);
+                                });
+  }
   SolveArgsT<T> a;
   std::memset(&a, 0, sizeof a);
   a.B = B; a.q = q; a.pose = base_pose; a.twist = base_twist; a.tpose = target_pose; a.ttwist = target_twist;
   a.mask = stance_mask; a.mu = mu; a.normals = normals_world;
   a.grf = grf; a.tau = tau; a.flags = flags; a.netwrench = netwrench; a.wrench_out = wrench_out;
-  a.counter = ctx->d_counter; a.model = Typed<T>::model(ctx); a.params = Typed<T>::params(ctx); a.params64 = ctx->d_params;
-  return Typed<T>::template launch<1>(ctx, a, static_cast<cudaStream_t>(stream));
-}
-
-// ---- host-pointer entry points: copy in, solve, copy out, synchronise.
-// Large batches are cut into chunks of kChunk states that flow through kPipe streams, so that the H2D
-// copy of chunk i+1, the kernel of chunk i and the D2H copy of chunk i-1 overlap (PCIe is full duplex).
-// The arrays are SoA with row pitch B, so a chunk is a column range: one 2-D copy per array.
-template <typename T> struct HostRow { const T* h; int rows; };   // input array (may be null) and its component count
-template <typename T> struct HostOut { T* h; int rows; };
-
-template <typename T>
-int host_pipeline_chunks(qlb_context* ctx, size_t B, bool state_mode, const HostRow<T>* in, int nin, const uint8_t* mask,
-                      const HostOut<T>* out, int nout, uint32_t* flags) {
-  int rc = QLB_OK;
-  const size_t cap = ctx->cap;
-  const size_t nchunks = (B + cap - 1) / cap;
-  for (size_t ci = 0; ci < nchunks; ci++) {
-    const int slot = (int)(ci % kPipe);
-    cudaStream_t st = ctx->pipe[slot];
-    const size_t b0 = ci * cap, n = (B - b0 < cap) ? (B - b0) : cap;
-    // the staging buffers are sized for FP64; the FP32 twins use the first half of each slot
-    T* din = reinterpret_cast<T*>(ctx->d_in + (size_t)slot * cap * kHostInRows);
-    T* dout = reinterpret_cast<T*>(ctx->d_out + (size_t)slot * cap * kHostOutRows);
-    uint8_t* dmask = ctx->d_mask + (size_t)slot * cap;
-    uint32_t* dflags = ctx->d_flags + (size_t)slot * cap;
-    const T* dptr_in[8];
-    size_t off = 0;
-    for (int k = 0; k < nin; k++) {
-      dptr_in[k] = nullptr;
-      if (in[k].h) {
-        dptr_in[k] = din + off;
-        QLB_CUDA(ctx, cudaMemcpy2DAsync(din + off, n * sizeof(T), in[k].h + b0, B * sizeof(T), n * sizeof(T), in[k].rows,
-                                        cudaMemcpyHostToDevice, st));
-      }
-      off += (size_t)in[k].rows * cap;   // fixed block sizes keep every block 16-byte aligned (cap % 16 == 0)
-    }
-    QLB_CUDA(ctx, cudaMemcpyAsync(dmask, mask + b0, n, cudaMemcpyHostToDevice, st));
-    T* dptr_out[4];
-    off = 0;
-    for (int k = 0; k < nout; k++) {
-      dptr_out[k] = out[k].h ? dout + off : nullptr;
-      off += (size_t)out[k].rows * cap;
-    }
-    if (!state_mode)
-      rc = solve_wrench_t<T>(ctx, n, dptr_in[0], dptr_in[1], dptr_in[2], dmask, dptr_in[3], dptr_in[4], dptr_out[0], dptr_out[1],
-                             dflags, dptr_out[2], st);
-    else
-      rc = solve_state_t<T>(ctx, n, dptr_in[0], dptr_in[1], dptr_in[2], dptr_in[3], dptr_in[4], dmask, dptr_in[5], dptr_in[6],
-                            dptr_out[0], dptr_out[1], dflags, dptr_out[2], dptr_out[3], st);
-    if (rc != QLB_OK) return rc;
-    for (int k = 0; k < nout; k++)
-      if (out[k].h)
-        QLB_CUDA(ctx, cudaMemcpy2DAsync(out[k].h + b0, B * sizeof(T), dptr_out[k], n * sizeof(T), n * sizeof(T), out[k].rows,
-                                        cudaMemcpyDeviceToHost, st));
-    QLB_CUDA(ctx, cudaMemcpyAsync(flags + b0, dflags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-  }
-  return QLB_OK;
-}
-
-
-template <typename T>
-int run_host_pipeline(qlb_context* ctx, size_t B, bool state_mode, const HostRow<T>* in, int nin, const uint8_t* mask,
-                      const HostOut<T>* out, int nout, uint32_t* flags) {
-  int rc = ensure_capacity(ctx, B);
-  if (rc != QLB_OK) return rc;
-  rc = host_pipeline_chunks<T>(ctx, B, state_mode, in, nin, mask, out, nout, flags);
-  // also on failure: no copy may still be reading or writing the caller's buffers when the call returns
-  for (int i = 0; i < kPipe; i++)
-    if (cudaStreamSynchronize(ctx->pipe[i]) != cudaSuccess && rc == QLB_OK) rc = cuda_fail(ctx, cudaGetLastError(), "cudaStreamSynchronize");
-  return rc;
-}
-
-template <typename T>
-int solve_wrench_host_t(qlb_context* ctx, size_t B, const T* q, const T* quat_wxyz, const T* wrench, const uint8_t* stance_mask,
-                        const T* mu, const T* normals_world, T* grf, T* tau, uint32_t* flags, T* netwrench) {
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (B == 0) return QLB_OK;
-  if (!q || !quat_wxyz || !wrench || !stance_mask || !grf || !tau || !flags) return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  const HostRow<T> in[5] = {{q, 12}, {quat_wxyz, 4}, {wrench, 6}, {mu, 4}, {normals_world, 12}};
-  const HostOut<T> out[3] = {{grf, 12}, {tau, 12}, {netwrench, 6}};
-  return run_host_pipeline<T>(ctx, B, false, in, 5, stance_mask, out, 3, flags);
-}
-
-template <typename T>
-int solve_state_host_t(qlb_context* ctx, size_t B, const T* q, const T* base_pose, const T* base_twist, const T* target_pose,
-                       const T* target_twist, const uint8_t* stance_mask, const T* mu, const T* normals_world, T* grf, T* tau,
-                       uint32_t* flags, T* netwrench, T* wrench_out) {
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (B == 0) return QLB_OK;
-  if (!q || !base_pose || !base_twist || !target_pose || !target_twist || !stance_mask || !grf || !tau || !flags)
-    return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  const HostRow<T> in[7] = {{q, 12}, {base_pose, 7}, {base_twist, 6}, {target_pose, 7}, {target_twist, 6}, {mu, 4}, {normals_world, 12}};
-  const HostOut<T> out[4] = {{grf, 12}, {tau, 12}, {netwrench, 6}, {wrench_out, 6}};
-  return run_host_pipeline<T>(ctx, B, true, in, 7, stance_mask, out, 4, flags);
+  a.model = Typed<T>::model(ctx); a.params = Typed<T>::params(ctx); a.params64 = ctx->d_params;
+  return launch_solve<T, 1>(ctx, a, static_cast<cudaStream_t>(stream));
 }
 
 }  // namespace
@@ -884,13 +909,13 @@ int qlb_solve_wrench(qlb_context* ctx, size_t B, const double* q, const double* 
                      const uint8_t* stance_mask, const double* mu, const double* normals_world, double* grf,
                      double* tau, uint32_t* flags, double* netwrench, void* stream) {
   QLB_GUARD(ctx);
-  return solve_wrench_t<double>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, stream);
+  return solve_wrench_t<double>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, stream, false);
 }
 int qlb_solve_wrench_f32(qlb_context* ctx, size_t B, const float* q, const float* quat_wxyz, const float* wrench,
                          const uint8_t* stance_mask, const float* mu, const float* normals_world, float* grf, float* tau,
                          uint32_t* flags, float* netwrench, void* stream) {
   QLB_GUARD(ctx);
-  return solve_wrench_t<float>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, stream);
+  return solve_wrench_t<float>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, stream, false);
 }
 int qlb_solve_state(qlb_context* ctx, size_t B, const double* q, const double* base_pose, const double* base_twist,
                     const double* target_pose, const double* target_twist, const uint8_t* stance_mask,
@@ -898,7 +923,7 @@ int qlb_solve_state(qlb_context* ctx, size_t B, const double* q, const double* b
                     double* netwrench, double* wrench_out, void* stream) {
   QLB_GUARD(ctx);
   return solve_state_t<double>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world, grf,
-                               tau, flags, netwrench, wrench_out, stream);
+                               tau, flags, netwrench, wrench_out, stream, false);
 }
 int qlb_solve_state_f32(qlb_context* ctx, size_t B, const float* q, const float* base_pose, const float* base_twist,
                         const float* target_pose, const float* target_twist, const uint8_t* stance_mask, const float* mu,
@@ -906,35 +931,35 @@ int qlb_solve_state_f32(qlb_context* ctx, size_t B, const float* q, const float*
                         float* wrench_out, void* stream) {
   QLB_GUARD(ctx);
   return solve_state_t<float>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world, grf,
-                              tau, flags, netwrench, wrench_out, stream);
+                              tau, flags, netwrench, wrench_out, stream, false);
 }
 int qlb_solve_wrench_host(qlb_context* ctx, size_t B, const double* q, const double* quat_wxyz, const double* wrench,
                           const uint8_t* stance_mask, const double* mu, const double* normals_world, double* grf,
                           double* tau, uint32_t* flags, double* netwrench) {
   QLB_GUARD(ctx);
-  return solve_wrench_host_t<double>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench);
+  return solve_wrench_t<double>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, nullptr, true);
 }
 int qlb_solve_wrench_f32_host(qlb_context* ctx, size_t B, const float* q, const float* quat_wxyz, const float* wrench,
                               const uint8_t* stance_mask, const float* mu, const float* normals_world, float* grf, float* tau,
                               uint32_t* flags, float* netwrench) {
   QLB_GUARD(ctx);
-  return solve_wrench_host_t<float>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench);
+  return solve_wrench_t<float>(ctx, B, q, quat_wxyz, wrench, stance_mask, mu, normals_world, grf, tau, flags, netwrench, nullptr, true);
 }
 int qlb_solve_state_host(qlb_context* ctx, size_t B, const double* q, const double* base_pose, const double* base_twist,
                          const double* target_pose, const double* target_twist, const uint8_t* stance_mask,
                          const double* mu, const double* normals_world, double* grf, double* tau, uint32_t* flags,
                          double* netwrench, double* wrench_out) {
   QLB_GUARD(ctx);
-  return solve_state_host_t<double>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world,
-                                    grf, tau, flags, netwrench, wrench_out);
+  return solve_state_t<double>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world,
+                               grf, tau, flags, netwrench, wrench_out, nullptr, true);
 }
 int qlb_solve_state_f32_host(qlb_context* ctx, size_t B, const float* q, const float* base_pose, const float* base_twist,
                              const float* target_pose, const float* target_twist, const uint8_t* stance_mask, const float* mu,
                              const float* normals_world, float* grf, float* tau, uint32_t* flags, float* netwrench,
                              float* wrench_out) {
   QLB_GUARD(ctx);
-  return solve_state_host_t<float>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world,
-                                   grf, tau, flags, netwrench, wrench_out);
+  return solve_state_t<float>(ctx, B, q, base_pose, base_twist, target_pose, target_twist, stance_mask, mu, normals_world,
+                              grf, tau, flags, netwrench, wrench_out, nullptr, true);
 }
 
 int qlb_leg_kinematics(qlb_context* ctx, size_t B, const double* q, const double* quat_wxyz, double* foot, double* jac,
@@ -944,15 +969,8 @@ int qlb_leg_kinematics(qlb_context* ctx, size_t B, const double* q, const double
   if (B == 0) return QLB_OK;
   if (!q) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  const unsigned long long total = (unsigned long long)B * 4ull;
-  const unsigned threads = 128;
-  const unsigned long long blocks = (total + threads - 1) / threads;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_kinematics_kernel<<<(unsigned)blocks, threads, 0, static_cast<cudaStream_t>(stream)>>>(
-      B, q, quat_wxyz, foot, jac, gravity_tau, ctx->d_model, ctx->d_params);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  return launch_items(ctx, B * 4ull, 128, static_cast<cudaStream_t>(stream), qlb_kinematics_kernel, (unsigned long long)B, q,
+                      quat_wxyz, foot, jac, gravity_tau, ctx->d_model, ctx->d_params, nullptr, nullptr);
 }
 
 int qlb_pack_robot_states(qlb_context* ctx, size_t B, const qlb_robot_state_record* records, double* q, double* base_pose,
@@ -963,13 +981,8 @@ int qlb_pack_robot_states(qlb_context* ctx, size_t B, const qlb_robot_state_reco
   if (B == 0) return QLB_OK;
   if (!records || !aligned16(records)) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  const unsigned long long blocks = ((unsigned long long)B + kPackTile - 1) / kPackTile;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_pack_kernel<<<(unsigned)blocks, kPackTile, 0, static_cast<cudaStream_t>(stream)>>>(B, records, q, base_pose, base_twist,
-                                                                                       stance_mask, normals_world);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  return launch_items(ctx, B, kPackTile, static_cast<cudaStream_t>(stream), qlb_pack_kernel, (unsigned long long)B, records, q,
+                      base_pose, base_twist, stance_mask, normals_world);
 }
 
 int qlb_feet_in_world(qlb_context* ctx, size_t B, const double* q, const double* base_pose, double* feet_world, void* stream) {
@@ -978,15 +991,8 @@ int qlb_feet_in_world(qlb_context* ctx, size_t B, const double* q, const double*
   if (B == 0) return QLB_OK;
   if (!q || !base_pose || !feet_world) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  const unsigned long long total = (unsigned long long)B * 4ull;
-  const unsigned threads = 128;
-  const unsigned long long blocks = (total + threads - 1) / threads;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_kinematics_kernel<<<(unsigned)blocks, threads, 0, static_cast<cudaStream_t>(stream)>>>(
-      B, q, nullptr, nullptr, nullptr, nullptr, ctx->d_model, ctx->d_params, base_pose, feet_world);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  return launch_items(ctx, B * 4ull, 128, static_cast<cudaStream_t>(stream), qlb_kinematics_kernel, (unsigned long long)B, q,
+                      nullptr, nullptr, nullptr, nullptr, ctx->d_model, ctx->d_params, base_pose, feet_world);
 }
 
 int qlb_default_swing_params(qlb_swing_params* p) {
@@ -1026,28 +1032,67 @@ int qlb_set_limb_dynamics(qlb_context* ctx, const qlb_limb_dynamics legs[QLB_NUM
   return QLB_OK;
 }
 
-int qlb_swing_leg_torques(qlb_context* ctx, size_t B, const double* q, const double* qd, const double* qdd,
-                          const double* foot_target_position, const double* foot_target_velocity,
-                          const qlb_swing_params* params, double* tau, void* stream) {
-  QLB_GUARD(ctx);
+extern "C++" {
+namespace {
+// The swing-leg arguments every caller fills alike; the caller sets qdd, or qd_front / ld_front / inv_window.
+template <typename T>
+void fill_swing(SwingArgsT<T>& s, const qlb_context* ctx, const qlb_swing_params& p, size_t B, const T* q, const T* qd,
+                const T* ptarget, const T* vtarget, T* tau) {
+  std::memset(&s, 0, sizeof s);
+  s.B = B; s.q = q; s.qd = qd; s.ptarget = ptarget; s.vtarget = vtarget; s.tau = tau;
+  for (int k = 0; k < 3; k++) { s.gravity[k] = (T)p.gravity[k]; s.kp[k] = (T)p.kp[k]; s.kd[k] = (T)p.kd[k]; }
+  s.acc_scale = (T)p.acceleration_scale;
+  s.dyn = Typed<T>::limb(ctx); s.model = Typed<T>::model(ctx);
+}
+
+// qlb_swing_leg_torques and its host twin: checks, then one launch on `stream`, or chunks of the staging capacity on
+// the context stream
+int swing_leg_torques(qlb_context* ctx, size_t B, const double* q, const double* qd, const double* qdd,
+                      const double* foot_target_position, const double* foot_target_velocity, const qlb_swing_params* params,
+                      double* tau, void* stream, bool host) {
   if (!ctx) return QLB_ERR_NOT_INITIALISED;
   if (!ctx->have_limb) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
   if (B == 0) return QLB_OK;
   if (!q || !qd || !qdd || !params || !tau) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
+  if (host) {
+    QLB_TRY(reserve_soa(ctx, B));
+    const size_t cap = ctx->cap;   // the input staging area holds kPipe * cap * 54 doubles >= 5 * 12 * cap
+    static_assert(kPipe * kHostInRows >= 60 && kPipe * kHostOutRows >= 12, "staging too small for the swing-leg arrays");
+    const SoaSlot s = soa_slot(ctx, 0);
+    const double* src[5] = {q, qd, qdd, foot_target_position, foot_target_velocity};
+    return for_chunks(ctx, B, cap, false, [&](size_t b0, size_t n, int, cudaStream_t st) -> int {
+      const double* dptr[5];
+      for (int k = 0; k < 5; k++) {
+        double* d = s.in + (size_t)k * 12 * cap;
+        dptr[k] = src[k] ? d : nullptr;
+        QLB_TRY(rows_to_device(ctx, d, src[k], 12, b0, n, B, st));
+      }
+      QLB_TRY(swing_leg_torques(ctx, n, dptr[0], dptr[1], dptr[2], dptr[3], dptr[4], params, s.out, st, false));
+      return rows_to_host(ctx, tau, s.out, 12, b0, n, B, st);
+    });
+  }
   SwingArgs a;
-  std::memset(&a, 0, sizeof a);
-  a.B = B; a.q = q; a.qd = qd; a.qdd = qdd; a.ptarget = foot_target_position; a.vtarget = foot_target_velocity; a.tau = tau;
-  for (int c = 0; c < 3; c++) { a.gravity[c] = params->gravity[c]; a.kp[c] = params->kp[c]; a.kd[c] = params->kd[c]; }
-  a.acc_scale = params->acceleration_scale;
-  a.dyn = ctx->d_limb; a.model = ctx->d_model;
-  const unsigned long long total = (unsigned long long)B * 4ull;
-  const unsigned long long blocks = (total + 127) / 128;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_swing_kernel<<<(unsigned)blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(a);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  fill_swing(a, ctx, *params, B, q, qd, foot_target_position, foot_target_velocity, tau);
+  a.qdd = qdd;
+  return launch_items(ctx, B * 4ull, 128, static_cast<cudaStream_t>(stream), qlb_swing_kernel, a);
+}
+}  // namespace
+}  // extern "C++"
+
+int qlb_swing_leg_torques(qlb_context* ctx, size_t B, const double* q, const double* qd, const double* qdd,
+                          const double* foot_target_position, const double* foot_target_velocity,
+                          const qlb_swing_params* params, double* tau, void* stream) {
+  QLB_GUARD(ctx);
+  return swing_leg_torques(ctx, B, q, qd, qdd, foot_target_position, foot_target_velocity, params, tau, stream, false);
+}
+
+// HOST pointers: staged through the context's SoA staging in chunks, on the context stream; synchronises.
+int qlb_swing_leg_torques_host(qlb_context* ctx, size_t B, const double* q, const double* qd, const double* qdd,
+                               const double* foot_target_position, const double* foot_target_velocity,
+                               const qlb_swing_params* params, double* tau) {
+  QLB_GUARD(ctx);
+  return swing_leg_torques(ctx, B, q, qd, qdd, foot_target_position, foot_target_velocity, params, tau, nullptr, true);
 }
 
 int qlb_swing_leg_torques_from_queue(qlb_context* ctx, size_t B, const double* q, const double* qd_back, const double* qd_front,
@@ -1060,19 +1105,9 @@ int qlb_swing_leg_torques_from_queue(qlb_context* ctx, size_t B, const double* q
   if (!q || !qd_back || !qd_front || !params || !tau || !(period > 0.0)) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
   SwingArgs a;
-  std::memset(&a, 0, sizeof a);
-  a.B = B; a.q = q; a.qd = qd_back; a.qdd = nullptr; a.qd_front = qd_front; a.ld_front = B; a.inv_window = 1.0 / (10.0 * period);
-  a.ptarget = foot_target_position; a.vtarget = foot_target_velocity; a.tau = tau;
-  for (int c = 0; c < 3; c++) { a.gravity[c] = params->gravity[c]; a.kp[c] = params->kp[c]; a.kd[c] = params->kd[c]; }
-  a.acc_scale = params->acceleration_scale;
-  a.dyn = ctx->d_limb; a.model = ctx->d_model;
-  const unsigned long long total = (unsigned long long)B * 4ull;
-  const unsigned long long blocks = (total + 127) / 128;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_swing_kernel<<<(unsigned)blocks, 128, 0, static_cast<cudaStream_t>(stream)>>>(a);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  fill_swing(a, ctx, *params, B, q, qd_back, foot_target_position, foot_target_velocity, tau);
+  a.qd_front = qd_front; a.ld_front = B; a.inv_window = 1.0 / (10.0 * period);
+  return launch_items(ctx, B * 4ull, 128, static_cast<cudaStream_t>(stream), qlb_swing_kernel, a);
 }
 
 int qlb_contact_fsm(qlb_context* ctx, size_t B, const uint8_t* desired_stance_mask, const uint8_t* footstep_mask,
@@ -1082,13 +1117,8 @@ int qlb_contact_fsm(qlb_context* ctx, size_t B, const uint8_t* desired_stance_ma
   if (B == 0) return QLB_OK;
   if (!desired_stance_mask || !contact_mask || !phase || !limb_state) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  const unsigned long long blocks = ((unsigned long long)B + 255) / 256;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_contact_fsm_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(B, desired_stance_mask, footstep_mask,
-                                                                                         contact_mask, phase, limb_state, stance_mask);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  return launch_items(ctx, B, 256, static_cast<cudaStream_t>(stream), qlb_contact_fsm_kernel, (unsigned long long)B,
+                      desired_stance_mask, footstep_mask, contact_mask, phase, limb_state, stance_mask);
 }
 
 int qlb_friction_margins(qlb_context* ctx, size_t B, const double* grf, const double* quat_wxyz, const uint8_t* stance_mask,
@@ -1098,133 +1128,67 @@ int qlb_friction_margins(qlb_context* ctx, size_t B, const double* grf, const do
   if (B == 0) return QLB_OK;
   if (!grf || !quat_wxyz || !stance_mask || !margin) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  const unsigned long long blocks = ((unsigned long long)B + 255) / 256;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_friction_margin_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(B, grf, quat_wxyz, stance_mask, mu,
-                                                                                             normals_world, ctx->d_params, margin, min_normal);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
-}
-
-// HOST pointers: staged through the context's pipeline buffers in chunks, on the context stream; synchronises.
-int qlb_swing_leg_torques_host(qlb_context* ctx, size_t B, const double* q, const double* qd, const double* qdd,
-                               const double* foot_target_position, const double* foot_target_velocity,
-                               const qlb_swing_params* params, double* tau) {
-  QLB_GUARD(ctx);
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (!ctx->have_limb) return QLB_ERR_NOT_INITIALISED;
-  if (B == 0) return QLB_OK;
-  if (!q || !qd || !qdd || !params || !tau) return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, B);
-  if (rc != QLB_OK) return rc;
-  const size_t cap = ctx->cap;   // the input staging area holds kPipe * cap * 54 doubles >= 5 * 12 * cap
-  static_assert(kPipe * kHostInRows >= 60 && kPipe * kHostOutRows >= 12, "staging too small for the swing-leg arrays");
-  const double* src[5] = {q, qd, qdd, foot_target_position, foot_target_velocity};
-  for (size_t b0 = 0; b0 < B; b0 += cap) {
-    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
-    const double* dptr[5];
-    for (int k = 0; k < 5; k++) {
-      dptr[k] = nullptr;
-      if (!src[k]) continue;
-      double* d = ctx->d_in + (size_t)k * 12 * cap;
-      dptr[k] = d;
-      QLB_CUDA(ctx, cudaMemcpy2DAsync(d, n * sizeof(double), src[k] + b0, B * sizeof(double), n * sizeof(double), 12,
-                                      cudaMemcpyHostToDevice, ctx->stream));
-    }
-    rc = qlb_swing_leg_torques(ctx, n, dptr[0], dptr[1], dptr[2], dptr[3], dptr[4], params, ctx->d_out, ctx->stream);
-    if (rc != QLB_OK) { cudaStreamSynchronize(ctx->stream); return rc; }
-    QLB_CUDA(ctx, cudaMemcpy2DAsync(tau + b0, B * sizeof(double), ctx->d_out, n * sizeof(double), n * sizeof(double), 12,
-                                    cudaMemcpyDeviceToHost, ctx->stream));
-    QLB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  }
-  return QLB_OK;
+  return launch_items(ctx, B, 256, static_cast<cudaStream_t>(stream), qlb_friction_margin_kernel, (unsigned long long)B, grf,
+                      quat_wxyz, stance_mask, mu, normals_world, ctx->d_params, margin, min_normal);
 }
 
 namespace {
 // one chunk of records on one stream: unpack, solve, pack (device pointers; `slot` selects the SoA staging area)
 int records_chunk(qlb_context* ctx, size_t n, const qlb_wrench_record* d_in, qlb_result_record* d_out, int slot, cudaStream_t st) {
   const size_t cap = ctx->cap;
-  double* din = ctx->d_in + (size_t)slot * cap * kHostInRows;
-  double* dout = ctx->d_out + (size_t)slot * cap * kHostOutRows;
-  uint8_t* dmask = ctx->d_mask + (size_t)slot * cap;
-  uint32_t* dflags = ctx->d_flags + (size_t)slot * cap;
-  double* q = din; double* quat = din + 12 * cap; double* wrench = din + 16 * cap; double* mu = din + 22 * cap;
-  double* grf = dout; double* tau = dout + 12 * cap; double* net = dout + 24 * cap;
-  const unsigned blocks = (unsigned)((n + kRecTile - 1) / kRecTile);
+  const SoaSlot s = soa_slot(ctx, slot);
+  double* q = s.in; double* quat = s.in + 12 * cap; double* wrench = s.in + 16 * cap; double* mu = s.in + 22 * cap;
+  double* grf = s.out; double* tau = s.out + 12 * cap; double* net = s.out + 24 * cap;
   // the SoA staging rows have pitch n inside this chunk
-  qlb_unpack_records_kernel<<<blocks, kRecTile, 0, st>>>(n, d_in, q, quat, wrench, mu, dmask);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  const int rc = solve_wrench_t<double>(ctx, n, q, quat, wrench, dmask, mu, nullptr, grf, tau, dflags, net, st);
-  if (rc != QLB_OK) return rc;
-  qlb_pack_results_kernel<<<blocks, kRecTile, 0, st>>>(n, grf, tau, net, dflags, d_out);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  QLB_TRY(launch_items(ctx, n, kRecTile, st, qlb_unpack_records_kernel, (unsigned long long)n, d_in, q, quat, wrench, mu, s.mask));
+  QLB_TRY(solve_wrench_t<double>(ctx, n, q, quat, wrench, s.mask, mu, nullptr, grf, tau, s.flags, net, st, false));
+  return launch_items(ctx, n, kRecTile, st, qlb_pack_results_kernel, (unsigned long long)n, grf, tau, net, s.flags, d_out);
 }
 
-int records_host_chunks(qlb_context* ctx, size_t B, const qlb_wrench_record* in, qlb_result_record* out) {
+// qlb_solve_records and its host twin: checks, then the chunks on `stream` (one staging area: the caller's arrays are
+// already on the device, nothing to overlap), or on the pipeline with one 1-D copy per chunk and direction
+int solve_records(qlb_context* ctx, size_t B, const qlb_wrench_record* records, qlb_result_record* results, void* stream,
+                  bool host) {
+  if (!ctx) return QLB_ERR_NOT_INITIALISED;
+  if (B == 0) return QLB_OK;
+  if (!records || !results) return QLB_ERR_INVALID_ARGUMENT;
+  DeviceGuard guard(ctx->device);
+  QLB_TRY(reserve_soa(ctx, B));
   const size_t cap = ctx->cap;
-  const size_t nchunks = (B + cap - 1) / cap;
-  for (size_t ci = 0; ci < nchunks; ci++) {
-    const int slot = (int)(ci % kPipe);
-    cudaStream_t st = ctx->pipe[slot];
-    const size_t b0 = ci * cap, n = (B - b0 < cap) ? (B - b0) : cap;
-    unsigned char* base = ctx->d_rec + (size_t)slot * cap * (sizeof(qlb_wrench_record) + sizeof(qlb_result_record));
-    qlb_wrench_record* d_in = reinterpret_cast<qlb_wrench_record*>(base);
-    qlb_result_record* d_out = reinterpret_cast<qlb_result_record*>(base + cap * sizeof(qlb_wrench_record));
-    QLB_CUDA(ctx, cudaMemcpyAsync(d_in, in + b0, n * sizeof(qlb_wrench_record), cudaMemcpyHostToDevice, st));
-    const int rc = records_chunk(ctx, n, d_in, d_out, slot, st);
-    if (rc != QLB_OK) return rc;
-    QLB_CUDA(ctx, cudaMemcpyAsync(out + b0, d_out, n * sizeof(qlb_result_record), cudaMemcpyDeviceToHost, st));
+  if (host) {
+    constexpr size_t per_state = sizeof(qlb_wrench_record) + sizeof(qlb_result_record);
+    QLB_TRY(reserve(ctx, ctx->rec, kPipe * cap * per_state));
+    return for_chunks(ctx, B, cap, true, [&](size_t b0, size_t n, int slot, cudaStream_t st) -> int {
+      unsigned char* base = ctx->rec.p + (size_t)slot * cap * per_state;
+      qlb_wrench_record* d_in = reinterpret_cast<qlb_wrench_record*>(base);
+      qlb_result_record* d_out = reinterpret_cast<qlb_result_record*>(base + cap * sizeof(qlb_wrench_record));
+      QLB_CUDA(ctx, cudaMemcpyAsync(d_in, records + b0, n * sizeof(qlb_wrench_record), cudaMemcpyHostToDevice, st));
+      QLB_TRY(records_chunk(ctx, n, d_in, d_out, slot, st));
+      QLB_CUDA(ctx, cudaMemcpyAsync(results + b0, d_out, n * sizeof(qlb_result_record), cudaMemcpyDeviceToHost, st));
+      return QLB_OK;
+    });
   }
-  return QLB_OK;
+  // the only asynchronous user of the SoA staging: ordered after the previous one, and recorded (on failure too) for
+  // the next user to wait on
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  QLB_CUDA(ctx, cudaStreamWaitEvent(st, ctx->soa_free, 0));
+  int rc = QLB_OK;
+  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap)
+    rc = records_chunk(ctx, B - b0 < cap ? B - b0 : cap, records + b0, results + b0, 0, st);
+  const cudaError_t e = cudaEventRecord(ctx->soa_free, st);
+  if (e != cudaSuccess && rc == QLB_OK) rc = cuda_fail(ctx, e, "cudaEventRecord");
+  return rc;
 }
 }  // namespace
 
 int qlb_solve_records(qlb_context* ctx, size_t B, const qlb_wrench_record* records, qlb_result_record* results, void* stream) {
   QLB_GUARD(ctx);
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (B == 0) return QLB_OK;
-  if (!records || !results) return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, B);
-  if (rc != QLB_OK) return rc;
-  const size_t cap = ctx->cap;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  // one staging area, chunks in stream order (the caller's arrays are already on the device: nothing to overlap)
-  for (size_t b0 = 0; b0 < B; b0 += cap) {
-    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
-    rc = records_chunk(ctx, n, records + b0, results + b0, 0, st);
-    if (rc != QLB_OK) return rc;
-  }
-  return QLB_OK;
+  return solve_records(ctx, B, records, results, stream, false);
 }
 
 int qlb_solve_records_host(qlb_context* ctx, size_t B, const qlb_wrench_record* records, qlb_result_record* results) {
   QLB_GUARD(ctx);
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (B == 0) return QLB_OK;
-  if (!records || !results) return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, B);
-  if (rc != QLB_OK) return rc;
-  if (ctx->rec_cap < ctx->cap) {
-    QLB_CUDA(ctx, cudaDeviceSynchronize());
-    cudaFree(ctx->d_rec);
-    ctx->d_rec = nullptr; ctx->rec_cap = 0;
-    if (cudaMalloc(&ctx->d_rec, (size_t)kPipe * ctx->cap * (sizeof(qlb_wrench_record) + sizeof(qlb_result_record))) != cudaSuccess) {
-      cudaGetLastError();
-      return QLB_ERR_ALLOC;
-    }
-    ctx->rec_cap = ctx->cap;
-  }
-  rc = records_host_chunks(ctx, B, records, results);
-  for (int i = 0; i < kPipe; i++)
-    if (cudaStreamSynchronize(ctx->pipe[i]) != cudaSuccess && rc == QLB_OK) rc = cuda_fail(ctx, cudaGetLastError(), "cudaStreamSynchronize");
-  return rc;
+  return solve_records(ctx, B, records, results, nullptr, true);
 }
 
 int qlb_preview_plan_host(qlb_context* ctx, size_t B, const qlb_robot_state_record* records, const double mu[4],
@@ -1234,51 +1198,31 @@ int qlb_preview_plan_host(qlb_context* ctx, size_t B, const qlb_robot_state_reco
   if (B == 0) return QLB_OK;
   if (!records || !preview) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, B);
-  if (rc != QLB_OK) return rc;
+  QLB_TRY(reserve_soa(ctx, B));
   const size_t cap = ctx->cap;
   // per state: the input record, the result record, and SoA rows for feet (12), friction coefficients (4), margins (2)
-  const size_t per_state = sizeof(qlb_robot_state_record) + sizeof(qlb_preview_record) + 18 * sizeof(double);
-  if (ctx->prev_cap < cap) {
-    QLB_CUDA(ctx, cudaDeviceSynchronize());
-    cudaFree(ctx->d_prev);
-    ctx->d_prev = nullptr; ctx->prev_cap = 0;
-    if (cudaMalloc(&ctx->d_prev, cap * per_state) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
-    ctx->prev_cap = cap;
-  }
-  cudaStream_t st = ctx->stream;
-  qlb_robot_state_record* d_rec = reinterpret_cast<qlb_robot_state_record*>(ctx->d_prev);
-  qlb_preview_record* d_res = reinterpret_cast<qlb_preview_record*>(ctx->d_prev + cap * sizeof(qlb_robot_state_record));
-  double* extra = reinterpret_cast<double*>(ctx->d_prev + cap * (sizeof(qlb_robot_state_record) + sizeof(qlb_preview_record)));
-  double* feet = extra; double* dmu = extra + 12 * cap; double* margin = extra + 16 * cap; double* minn = extra + 17 * cap;
-  double* din = ctx->d_in; double* dout = ctx->d_out;
-  double* q = din; double* pose = din + 12 * cap; double* twist = din + 19 * cap; double* nrm = din + 25 * cap;
-  double* grf = dout; double* tau = dout + 12 * cap; double* net = dout + 24 * cap; double* wout = dout + 30 * cap;
-  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap) {
-    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
-    if (cudaMemcpyAsync(d_rec, records + b0, n * sizeof(qlb_robot_state_record), cudaMemcpyHostToDevice, st) != cudaSuccess) { rc = QLB_ERR_CUDA; break; }
-    rc = qlb_pack_robot_states(ctx, n, d_rec, q, pose, twist, ctx->d_mask, nrm, st);
-    if (rc == QLB_OK) rc = qlb_feet_in_world(ctx, n, q, pose, feet, st);
-    if (rc == QLB_OK && mu) {
-      qlb_fill_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, 4, dmu, mu[0], mu[1], mu[2], mu[3]);
-      ctx->launches++;
-    }
+  constexpr size_t per_state = sizeof(qlb_robot_state_record) + sizeof(qlb_preview_record) + 18 * sizeof(double);
+  QLB_TRY(reserve(ctx, ctx->prev, cap * per_state));
+  qlb_robot_state_record* d_rec = reinterpret_cast<qlb_robot_state_record*>(ctx->prev.p);
+  qlb_preview_record* d_res = reinterpret_cast<qlb_preview_record*>(ctx->prev.p + cap * sizeof(qlb_robot_state_record));
+  double* extra = reinterpret_cast<double*>(ctx->prev.p + cap * (sizeof(qlb_robot_state_record) + sizeof(qlb_preview_record)));
+  double* feet = extra; double* dmu = mu ? extra + 12 * cap : nullptr; double* margin = extra + 16 * cap; double* minn = extra + 17 * cap;
+  const SoaSlot s = soa_slot(ctx, 0);
+  double* q = s.in; double* pose = s.in + 12 * cap; double* twist = s.in + 19 * cap; double* nrm = s.in + 25 * cap;
+  double* grf = s.out; double* tau = s.out + 12 * cap; double* net = s.out + 24 * cap; double* wout = s.out + 30 * cap;
+  return for_chunks(ctx, B, cap, false, [&](size_t b0, size_t n, int, cudaStream_t st) -> int {
+    QLB_CUDA(ctx, cudaMemcpyAsync(d_rec, records + b0, n * sizeof(qlb_robot_state_record), cudaMemcpyHostToDevice, st));
+    QLB_TRY(qlb_pack_robot_states(ctx, n, d_rec, q, pose, twist, s.mask, nrm, st));
+    QLB_TRY(qlb_feet_in_world(ctx, n, q, pose, feet, st));
+    if (mu) QLB_TRY(launch_items(ctx, n, 256, st, qlb_fill_rows_kernel, (unsigned long long)n, 4, dmu, mu[0], mu[1], mu[2], mu[3]));
     // the planned state is feedback AND target: zero tracking error
-    if (rc == QLB_OK) rc = solve_state_t<double>(ctx, n, q, pose, twist, pose, twist, ctx->d_mask, mu ? dmu : nullptr, nrm, grf, tau,
-                                                  ctx->d_flags, net, wout, st);
-    if (rc == QLB_OK) rc = qlb_friction_margins(ctx, n, grf, pose + 3 * n, ctx->d_mask, mu ? dmu : nullptr, nrm, margin, minn, st);
-    if (rc == QLB_OK) {
-      qlb_pack_preview_kernel<<<(unsigned)((n + kPrevTile - 1) / kPrevTile), kPrevTile, 0, st>>>(n, feet, grf, tau, net, wout, margin, minn,
-                                                                                             ctx->d_flags, d_res);
-      ctx->launches++;
-      if (cudaGetLastError() != cudaSuccess) rc = QLB_ERR_CUDA;
-    }
-    if (rc == QLB_OK && cudaMemcpyAsync(preview + b0, d_res, n * sizeof(qlb_preview_record), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-    // the staging is reused by the next chunk
-    if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
-  }
-  if (rc == QLB_ERR_CUDA) cuda_fail(ctx, cudaGetLastError(), "qlb_preview_plan_host");
-  return rc;
+    QLB_TRY(solve_state_t<double>(ctx, n, q, pose, twist, pose, twist, s.mask, dmu, nrm, grf, tau, s.flags, net, wout, st, false));
+    QLB_TRY(qlb_friction_margins(ctx, n, grf, pose + 3 * n, s.mask, dmu, nrm, margin, minn, st));
+    QLB_TRY(launch_items(ctx, n, kPrevTile, st, qlb_pack_preview_kernel, (unsigned long long)n, feet, grf, tau, net, wout, margin,
+                         minn, s.flags, d_res));
+    QLB_CUDA(ctx, cudaMemcpyAsync(preview + b0, d_res, n * sizeof(qlb_preview_record), cudaMemcpyDeviceToHost, st));
+    return QLB_OK;
+  });
 }
 
 namespace {
@@ -1290,12 +1234,7 @@ int generate_common(qlb_context* ctx, int config, size_t B, uint64_t start, uint
   DeviceGuard guard(ctx->device);
   g.B = B; g.start = start; g.config = config;
   g.seed = seed ? seed : (0x5EED0000ull + (unsigned long long)config);
-  const unsigned long long blocks = ((unsigned long long)B + 255) / 256;
-  if (blocks > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
-  qlb_generate_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(g);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  return launch_items(ctx, B, 256, static_cast<cudaStream_t>(stream), qlb_generate_kernel, g);
 }
 }  // namespace
 
@@ -1395,15 +1334,43 @@ int qlb_stats_allreduce(qlb_context* ctx, void* nccl_comm, qlb_stats* stats, voi
   return QLB_OK;
 }
 
-int qlb_qp_dense(qlb_context* ctx, size_t B, int n, int m, int p, const double* G, const double* g0, const double* CE,
-                 const double* ce0, const double* CI, const double* ci0, double* x, double* cost, uint32_t* status,
-                 uint32_t* active, void* stream) {
-  QLB_GUARD(ctx);
+extern "C++" {
+namespace {
+// qlb_qp_dense and its host twin: checks, then one launch on `stream`, or one call on the context stream through the
+// context's staging
+int qp_dense(qlb_context* ctx, size_t B, int n, int m, int p, const double* G, const double* g0, const double* CE,
+             const double* ce0, const double* CI, const double* ci0, double* x, double* cost, uint32_t* status,
+             uint32_t* active, void* stream, bool host) {
   if (!ctx) return QLB_ERR_NOT_INITIALISED;
   if (n < 1 || n > kQpMaxN || m < 0 || m > kQpMaxM || p < 0 || p > kQpMaxP) return QLB_ERR_INVALID_ARGUMENT;
   if (B == 0) return QLB_OK;
   if (!G || !g0 || !x || !status || (p > 0 && (!CE || !ce0)) || (m > 0 && (!CI || !ci0))) return QLB_ERR_INVALID_ARGUMENT;
   DeviceGuard guard(ctx->device);
+  if (host) {
+    const size_t nin = (size_t)(n * n + n + n * p + p + n * m + m) * B, nout = (size_t)(n + 1) * B;
+    // grown on demand (a controller calls this every tick with the same shape)
+    QLB_TRY(reserve(ctx, ctx->qp, pow2_at_least((nin + nout) * sizeof(double) + 2 * B * sizeof(uint32_t), 4096)));
+    double* dG = reinterpret_cast<double*>(ctx->qp.p); double* dg = dG + (size_t)n * n * B; double* dCE = dg + (size_t)n * B;
+    double* dce = dCE + (size_t)n * p * B; double* dCI = dce + (size_t)p * B; double* dci = dCI + (size_t)n * m * B;
+    double* d_out = dG + nin;
+    uint32_t* d_u = reinterpret_cast<uint32_t*>(d_out + nout);
+    if (p == 0) CE = ce0 = nullptr;   // may be set; nothing to copy
+    if (m == 0) CI = ci0 = nullptr;
+    return for_chunks(ctx, B, B, false, [&](size_t, size_t, int, cudaStream_t st) -> int {
+      QLB_TRY(rows_to_device(ctx, dG, G, (size_t)n * n, 0, B, B, st));
+      QLB_TRY(rows_to_device(ctx, dg, g0, n, 0, B, B, st));
+      QLB_TRY(rows_to_device(ctx, dCE, CE, (size_t)n * p, 0, B, B, st));
+      QLB_TRY(rows_to_device(ctx, dce, ce0, p, 0, B, B, st));
+      QLB_TRY(rows_to_device(ctx, dCI, CI, (size_t)n * m, 0, B, B, st));
+      QLB_TRY(rows_to_device(ctx, dci, ci0, m, 0, B, B, st));
+      QLB_TRY(qp_dense(ctx, B, n, m, p, dG, dg, p ? dCE : nullptr, p ? dce : nullptr, m ? dCI : nullptr, m ? dci : nullptr,
+                       d_out, d_out + (size_t)n * B, d_u, d_u + B, st, false));
+      QLB_TRY(rows_to_host(ctx, x, d_out, n, 0, B, B, st));
+      QLB_TRY(rows_to_host(ctx, cost, d_out + (size_t)n * B, 1, 0, B, B, st));
+      QLB_TRY(rows_to_host(ctx, status, d_u, 1, 0, B, B, st));
+      return rows_to_host(ctx, active, d_u + B, 1, 0, B, B, st);
+    });
+  }
   QpDenseArgs a;
   a.B = B; a.n = n; a.m = m; a.p = p; a.G = G; a.g0 = g0; a.CE = CE; a.ce0 = ce0; a.CI = CI; a.ci0 = ci0;
   a.x = x; a.cost = cost; a.status = status; a.active = active;
@@ -1416,51 +1383,21 @@ int qlb_qp_dense(qlb_context* ctx, size_t B, int n, int m, int p, const double* 
   ctx->launches++;
   return QLB_OK;
 }
+}  // namespace
+}  // extern "C++"
+
+int qlb_qp_dense(qlb_context* ctx, size_t B, int n, int m, int p, const double* G, const double* g0, const double* CE,
+                 const double* ce0, const double* CI, const double* ci0, double* x, double* cost, uint32_t* status,
+                 uint32_t* active, void* stream) {
+  QLB_GUARD(ctx);
+  return qp_dense(ctx, B, n, m, p, G, g0, CE, ce0, CI, ci0, x, cost, status, active, stream, false);
+}
 
 int qlb_qp_dense_host(qlb_context* ctx, size_t B, int n, int m, int p, const double* G, const double* g0,
                       const double* CE, const double* ce0, const double* CI, const double* ci0, double* x, double* cost,
                       uint32_t* status, uint32_t* active) {
   QLB_GUARD(ctx);
-  if (!ctx) return QLB_ERR_NOT_INITIALISED;
-  if (n < 1 || n > kQpMaxN || m < 0 || m > kQpMaxM || p < 0 || p > kQpMaxP) return QLB_ERR_INVALID_ARGUMENT;
-  if (B == 0) return QLB_OK;
-  if (!G || !g0 || !x || !status || (p > 0 && (!CE || !ce0)) || (m > 0 && (!CI || !ci0))) return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(ctx->device);
-  cudaStream_t st = ctx->stream;
-  const size_t nin = (size_t)(n * n + n + n * p + p + n * m + m) * B, nout = (size_t)(n + 1) * B;
-  // staging owned by the context, grown on demand (a controller calls this every tick with the same shape)
-  const size_t need = (nin + nout) * sizeof(double) + 2 * B * sizeof(uint32_t);
-  if (ctx->qp_bytes < need) {
-    QLB_CUDA(ctx, cudaStreamSynchronize(st));
-    cudaFree(ctx->d_qp);
-    ctx->d_qp = nullptr; ctx->qp_bytes = 0;
-    size_t cap = 4096;
-    while (cap < need) cap *= 2;
-    if (cudaMalloc(&ctx->d_qp, cap) != cudaSuccess) { cudaGetLastError(); return QLB_ERR_ALLOC; }
-    ctx->qp_bytes = cap;
-  }
-  double* d_in = reinterpret_cast<double*>(ctx->d_qp);
-  double* d_out = d_in + nin;
-  uint32_t* d_u = reinterpret_cast<uint32_t*>(d_out + nout);
-  double* dG = d_in; double* dg = dG + (size_t)n * n * B; double* dCE = dg + (size_t)n * B; double* dce = dCE + (size_t)n * p * B;
-  double* dCI = dce + (size_t)p * B; double* dci = dCI + (size_t)n * m * B;
-  int rc = QLB_OK;
-  auto H2D = [&](double* d, const double* h, size_t cnt) {
-    if (cnt && rc == QLB_OK && cudaMemcpyAsync(d, h, cnt * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-  };
-  H2D(dG, G, (size_t)n * n * B); H2D(dg, g0, (size_t)n * B); H2D(dCE, CE, (size_t)n * p * B); H2D(dce, ce0, (size_t)p * B);
-  H2D(dCI, CI, (size_t)n * m * B); H2D(dci, ci0, (size_t)m * B);
-  if (rc == QLB_OK) rc = qlb_qp_dense(ctx, B, n, m, p, dG, dg, p ? dCE : nullptr, p ? dce : nullptr, m ? dCI : nullptr,
-                                       m ? dci : nullptr, d_out, d_out + (size_t)n * B, d_u, d_u + B, st);
-  if (rc == QLB_OK) {
-    if (cudaMemcpyAsync(x, d_out, (size_t)n * B * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-    if (cost && cudaMemcpyAsync(cost, d_out + (size_t)n * B, B * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-    if (cudaMemcpyAsync(status, d_u, B * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-    if (active && cudaMemcpyAsync(active, d_u + B, B * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = QLB_ERR_CUDA;
-  }
-  if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
-  if (rc == QLB_ERR_CUDA) cuda_fail(ctx, cudaGetLastError(), "qlb_qp_dense_host");
-  return rc;
+  return qp_dense(ctx, B, n, m, p, G, g0, CE, ce0, CI, ci0, x, cost, status, active, nullptr, true);
 }
 
 int qlb_measure_fp64_peak(qlb_context* ctx, double* tflops_out) {
@@ -1521,9 +1458,6 @@ int controller_tick(qlb_controller* c, size_t n, size_t b0, const T* q, const T*
                     const T* phase, const T* mu, const T* normals, const T* ptarget, const T* vtarget, T* command,
                     uint32_t* flags, T* grf, cudaStream_t st) {
   qlb_context* ctx = c->ctx;
-  const unsigned long long blocks_pro = ((unsigned long long)n + 255) / 256;
-  const unsigned long long blocks_epi = (4ull * n + 127) / 128;
-  if (blocks_epi > 0x7fffffffull) return QLB_ERR_BATCH_TOO_LARGE;
   const size_t ld = c->B;
   T* tau = reinterpret_cast<T*>(c->tau);
   TickArgsT<T> a;
@@ -1532,110 +1466,72 @@ int controller_tick(qlb_controller* c, size_t n, size_t b0, const T* q, const T*
   a.desired = desired; a.footstep = footstep; a.contact = contact; a.phase = phase; a.qd = qd;
   a.limb = c->limb + b0; a.refill = c->refill + b0; a.ring = c->ring + b0; a.stance = c->stance;
   a.flags = flags; a.tau = tau; a.efforts = c->efforts + b0; a.command = command; a.limit = c->p.effort_limit;
-  SwingArgsT<T>& s = a.swing;
-  s.B = n; s.q = q; s.qd = qd;
-  s.qd_front = c->ring + (size_t)((c->head + 1) % kTickRing) * 12 * ld + b0; s.ld_front = ld;
-  s.inv_window = (T)(1.0 / (10.0 * c->p.period));
-  s.ptarget = ptarget; s.vtarget = vtarget;
-  for (int k = 0; k < 3; k++) { s.gravity[k] = (T)c->p.swing.gravity[k]; s.kp[k] = (T)c->p.swing.kp[k]; s.kd[k] = (T)c->p.swing.kd[k]; }
-  s.acc_scale = (T)c->p.swing.acceleration_scale;
-  s.dyn = Typed<T>::limb(ctx); s.model = Typed<T>::model(ctx);
+  fill_swing<T>(a.swing, ctx, c->p.swing, n, q, qd, ptarget, vtarget, nullptr);
+  a.swing.qd_front = c->ring + (size_t)((c->head + 1) % kTickRing) * 12 * ld + b0; a.swing.ld_front = ld;
+  a.swing.inv_window = (T)(1.0 / (10.0 * c->p.period));
   QLB_CUDA(ctx, cudaStreamWaitEvent(st, c->reset_done, 0));
-  qlb_tick_prologue_kernel<T><<<(unsigned)blocks_pro, 256, 0, st>>>(a);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  const int rc = solve_state_t<T>(ctx, n, q, pose, twist, tpose, ttwist, c->stance, mu, normals,
-                                  grf ? grf : reinterpret_cast<T*>(c->grf), tau, flags, nullptr, nullptr, st);
-  if (rc != QLB_OK) return rc;
-  qlb_tick_epilogue_kernel<T><<<(unsigned)blocks_epi, 128, 0, st>>>(a);
-  QLB_CUDA(ctx, cudaGetLastError());
-  ctx->launches++;
-  return QLB_OK;
+  QLB_TRY(launch_items(ctx, n, 256, st, qlb_tick_prologue_kernel<T>, a));
+  QLB_TRY(solve_state_t<T>(ctx, n, q, pose, twist, tpose, ttwist, c->stance, mu, normals, grf ? grf : reinterpret_cast<T*>(c->grf),
+                           tau, flags, nullptr, nullptr, st, false));
+  return launch_items(ctx, 4ull * n, 128, st, qlb_tick_epilogue_kernel<T>, a);
 }
 
-bool controller_ready(const qlb_controller* c) { return c && c->ctx && c->ctx->have_limb; }
-
+// qlb_controller_update[_f32] and the host twins: checks, then one tick of the whole batch on `stream`, or chunks of the
+// context's staging capacity one after the other on the context stream (they share the controller's stance and tau
+// scratch, which is not offset by b0).  The staging is sized for FP64; the FP32 twin uses the same row offsets in
+// float, i.e. the first half.
 template <typename T>
 int controller_update_t(qlb_controller* c, const T* q, const T* qd, const T* base_pose, const T* base_twist,
                         const T* target_pose, const T* target_twist, const uint8_t* desired_stance_mask,
                         const uint8_t* footstep_mask, const uint8_t* contact_mask, const T* phase, const T* mu,
                         const T* normals_world, const T* foot_target_position, const T* foot_target_velocity, T* command,
-                        uint32_t* flags, T* grf, void* stream) {
+                        uint32_t* flags, T* grf, void* stream, bool host) {
   if (!c) return QLB_ERR_NOT_INITIALISED;
   QLB_GUARD(c->ctx);
-  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
-  if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
-      !phase || !command || !flags)
-    return QLB_ERR_INVALID_ARGUMENT;
-  DeviceGuard guard(c->ctx->device);
-  const int rc = controller_tick<T>(c, c->B, 0, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
-                                    footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                    foot_target_velocity, command, flags, grf, static_cast<cudaStream_t>(stream));
-  if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
-  return rc;
-}
-
-// HOST pointers: chunks of the context's staging capacity, one after the other on the context stream; synchronises.
-// The staging buffers are sized for FP64; the FP32 twin uses the same row offsets in float, i.e. the first half.
-template <typename T>
-int controller_update_host_t(qlb_controller* c, const T* q, const T* qd, const T* base_pose, const T* base_twist,
-                             const T* target_pose, const T* target_twist, const uint8_t* desired_stance_mask,
-                             const uint8_t* footstep_mask, const uint8_t* contact_mask, const T* phase, const T* mu,
-                             const T* normals_world, const T* foot_target_position, const T* foot_target_velocity,
-                             T* command, uint32_t* flags, T* grf) {
-  if (!c) return QLB_ERR_NOT_INITIALISED;
-  QLB_GUARD(c->ctx);
-  if (!controller_ready(c)) return QLB_ERR_NOT_INITIALISED;
+  if (!c->ctx || !c->ctx->have_limb) return QLB_ERR_NOT_INITIALISED;   // qlb_set_limb_dynamics first
   if (!q || !qd || !base_pose || !base_twist || !target_pose || !target_twist || !desired_stance_mask || !contact_mask ||
       !phase || !command || !flags)
     return QLB_ERR_INVALID_ARGUMENT;
   qlb_context* ctx = c->ctx;
   DeviceGuard guard(ctx->device);
-  int rc = ensure_capacity(ctx, c->B);
-  if (rc != QLB_OK) return rc;
-  const size_t B = c->B, cap = ctx->cap;
-  cudaStream_t st = ctx->stream;
-  T* const d_in = reinterpret_cast<T*>(ctx->d_in);
-  T* const d_out = reinterpret_cast<T*>(ctx->d_out);
-  // inputs: 94 rows in the input staging (kPipe * 54 rows of cap), outputs 24 rows, the three masks one row each
-  constexpr int kIn = 11, kOut = 2;
-  const T* src[kIn] = {q, qd, base_pose, base_twist, target_pose, target_twist, phase, mu, normals_world,
-                       foot_target_position, foot_target_velocity};
-  const int rows[kIn] = {12, 12, 7, 6, 7, 6, 4, 4, 12, 12, 12};
-  static_assert(kPipe * kHostInRows >= 94 && kPipe * kHostOutRows >= 24 && kPipe >= 3, "staging too small for a tick");
-  const uint8_t* msrc[3] = {desired_stance_mask, footstep_mask, contact_mask};
-  T* dst_out[kOut] = {command, grf};
-  for (size_t b0 = 0; b0 < B && rc == QLB_OK; b0 += cap) {
-    const size_t n = (B - b0 < cap) ? (B - b0) : cap;
-    const T* din[kIn];
-    size_t off = 0;
-    for (int k = 0; k < kIn && rc == QLB_OK; k++) {
-      din[k] = src[k] ? d_in + off : nullptr;
-      if (src[k] && cudaMemcpy2DAsync(d_in + off, n * sizeof(T), src[k] + b0, B * sizeof(T), n * sizeof(T), rows[k],
-                                      cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-      off += (size_t)rows[k] * cap;
-    }
-    const uint8_t* dmask[3];
-    for (int k = 0; k < 3 && rc == QLB_OK; k++) {
-      dmask[k] = msrc[k] ? ctx->d_mask + (size_t)k * cap : nullptr;
-      if (msrc[k] && cudaMemcpyAsync(ctx->d_mask + (size_t)k * cap, msrc[k] + b0, n, cudaMemcpyHostToDevice, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-    }
-    if (rc != QLB_OK) break;
-    T* dout[kOut] = {d_out, d_out + 12 * cap};
-    rc = controller_tick<T>(c, n, b0, din[0], din[1], din[2], din[3], din[4], din[5], dmask[0], dmask[1], dmask[2], din[6],
-                            din[7], din[8], din[9], din[10], dout[0], ctx->d_flags, dout[1], st);
-    for (int k = 0; k < kOut && rc == QLB_OK; k++)
-      if (dst_out[k] && cudaMemcpy2DAsync(dst_out[k] + b0, B * sizeof(T), dout[k], n * sizeof(T), n * sizeof(T), 12,
-                                          cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        rc = QLB_ERR_CUDA;
-    if (rc == QLB_OK && cudaMemcpyAsync(flags + b0, ctx->d_flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess)
-      rc = QLB_ERR_CUDA;
+  const size_t B = c->B;
+  int rc;
+  if (!host) {
+    rc = controller_tick<T>(c, B, 0, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask, footstep_mask,
+                            contact_mask, phase, mu, normals_world, foot_target_position, foot_target_velocity, command, flags,
+                            grf, static_cast<cudaStream_t>(stream));
+  } else {
+    QLB_TRY(reserve_soa(ctx, B));
+    const size_t cap = ctx->cap;
+    const SoaSlot s = soa_slot(ctx, 0);
+    // inputs: 94 rows in the input staging (kPipe * 54 rows of cap), outputs 24 rows, the three masks one row each
+    constexpr int kIn = 11, kOut = 2;
+    const T* src[kIn] = {q, qd, base_pose, base_twist, target_pose, target_twist, phase, mu, normals_world,
+                         foot_target_position, foot_target_velocity};
+    const int rows[kIn] = {12, 12, 7, 6, 7, 6, 4, 4, 12, 12, 12};
+    static_assert(kPipe * kHostInRows >= 94 && kPipe * kHostOutRows >= 24 && kPipe >= 3, "staging too small for a tick");
+    const uint8_t* msrc[3] = {desired_stance_mask, footstep_mask, contact_mask};
+    T* const dst_out[kOut] = {command, grf};
+    T* const dout[kOut] = {reinterpret_cast<T*>(s.out), reinterpret_cast<T*>(s.out) + 12 * cap};
+    rc = for_chunks(ctx, B, cap, false, [&](size_t b0, size_t n, int, cudaStream_t st) -> int {
+      const T* din[kIn];
+      T* d = reinterpret_cast<T*>(s.in);
+      for (int k = 0; k < kIn; d += (size_t)rows[k] * cap, k++) {
+        din[k] = src[k] ? d : nullptr;
+        QLB_TRY(rows_to_device(ctx, d, src[k], rows[k], b0, n, B, st));
+      }
+      const uint8_t* dmask[3];
+      for (int k = 0; k < 3; k++) {
+        dmask[k] = msrc[k] ? s.mask + (size_t)k * cap : nullptr;
+        if (msrc[k]) QLB_CUDA(ctx, cudaMemcpyAsync(s.mask + (size_t)k * cap, msrc[k] + b0, n, cudaMemcpyHostToDevice, st));
+      }
+      QLB_TRY(controller_tick<T>(c, n, b0, din[0], din[1], din[2], din[3], din[4], din[5], dmask[0], dmask[1], dmask[2], din[6],
+                                 din[7], din[8], din[9], din[10], dout[0], s.flags, dout[1], st));
+      for (int k = 0; k < kOut; k++) QLB_TRY(rows_to_host(ctx, dst_out[k], dout[k], 12, b0, n, B, st));
+      QLB_CUDA(ctx, cudaMemcpyAsync(flags + b0, s.flags, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+      return QLB_OK;
+    });
   }
-  // also on failure: no copy may still be reading or writing the caller's buffers when the call returns
-  if (cudaStreamSynchronize(st) != cudaSuccess && rc == QLB_OK) rc = QLB_ERR_CUDA;
-  if (rc == QLB_ERR_CUDA) return cuda_fail(ctx, cudaGetLastError(), "qlb_controller_update_host");
   if (rc == QLB_OK) c->head = (c->head + 1) % kTickRing;
   return rc;
 }
@@ -1714,11 +1610,8 @@ int qlb_controller_reset(qlb_controller* c, const uint8_t* reset_mask, void* str
   if (!c) return QLB_ERR_NOT_INITIALISED;
   QLB_GUARD(c->ctx);
   DeviceGuard guard(c->ctx->device);
-  const unsigned long long blocks = ((unsigned long long)c->B + 255) / 256;
-  qlb_tick_reset_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(c->B, reset_mask, c->limb, c->efforts,
-                                                                                         c->refill);
-  QLB_CUDA(c->ctx, cudaGetLastError());
-  c->ctx->launches++;
+  QLB_TRY(launch_items(c->ctx, c->B, 256, static_cast<cudaStream_t>(stream), qlb_tick_reset_kernel, (unsigned long long)c->B,
+                       reset_mask, c->limb, c->efforts, c->refill));
   QLB_CUDA(c->ctx, cudaEventRecord(c->reset_done, static_cast<cudaStream_t>(stream)));
   return QLB_OK;
 }
@@ -1731,7 +1624,7 @@ int qlb_controller_update(qlb_controller* c, const double* q, const double* qd, 
                           uint32_t* flags, double* grf, void* stream) {
   return controller_update_t<double>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
                                      footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                     foot_target_velocity, command, flags, grf, stream);
+                                     foot_target_velocity, command, flags, grf, stream, false);
 }
 int qlb_controller_update_f32(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
                               const float* base_twist, const float* target_pose, const float* target_twist,
@@ -1741,7 +1634,7 @@ int qlb_controller_update_f32(qlb_controller* c, const float* q, const float* qd
                               uint32_t* flags, float* grf, void* stream) {
   return controller_update_t<float>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
                                     footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                    foot_target_velocity, command, flags, grf, stream);
+                                    foot_target_velocity, command, flags, grf, stream, false);
 }
 int qlb_controller_update_host(qlb_controller* c, const double* q, const double* qd, const double* base_pose,
                                const double* base_twist, const double* target_pose, const double* target_twist,
@@ -1749,9 +1642,9 @@ int qlb_controller_update_host(qlb_controller* c, const double* q, const double*
                                const uint8_t* contact_mask, const double* phase, const double* mu,
                                const double* normals_world, const double* foot_target_position,
                                const double* foot_target_velocity, double* command, uint32_t* flags, double* grf) {
-  return controller_update_host_t<double>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
-                                          footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                          foot_target_velocity, command, flags, grf);
+  return controller_update_t<double>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                     footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                     foot_target_velocity, command, flags, grf, nullptr, true);
 }
 int qlb_controller_update_f32_host(qlb_controller* c, const float* q, const float* qd, const float* base_pose,
                                    const float* base_twist, const float* target_pose, const float* target_twist,
@@ -1759,9 +1652,9 @@ int qlb_controller_update_f32_host(qlb_controller* c, const float* q, const floa
                                    const uint8_t* contact_mask, const float* phase, const float* mu,
                                    const float* normals_world, const float* foot_target_position,
                                    const float* foot_target_velocity, float* command, uint32_t* flags, float* grf) {
-  return controller_update_host_t<float>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
-                                         footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
-                                         foot_target_velocity, command, flags, grf);
+  return controller_update_t<float>(c, q, qd, base_pose, base_twist, target_pose, target_twist, desired_stance_mask,
+                                    footstep_mask, contact_mask, phase, mu, normals_world, foot_target_position,
+                                    foot_target_velocity, command, flags, grf, nullptr, true);
 }
 
 int qlb_controller_get_state(const qlb_controller* c, uint8_t* limb_state, double* efforts, void* stream) {
