@@ -281,15 +281,17 @@ __device__ __forceinline__ void dbas_round(RoundState<creal>& q, const creal* b,
   }
 #pragma unroll
   for (int r = 0; r < 6; r++) r6[r] = quad_sum(r6[r]);
-  const bool pd = chol6_thread(N, rdg);
+  bool pd;
   if (Tol<creal>::refine) {
+    pd = chol6_thread(N, rdg);
     creal rhs6[6];
 #pragma unroll
     for (int r = 0; r < 6; r++) rhs6[r] = r6[r];
     solve6_thread(N, rdg, r6);
     refine6(N, rdg, v, al, cc.sinv, rhs6, r6);
   } else {
-    solve6_thread(N, rdg, r6);   // r6 <- t = S (b - A y+)
+    pd = ldl6_thread(N, rdg);
+    ldl6_solve(N, rdg, r6);   // r6 <- t = S (b - A y+)
   }
   // ---- y+ and the multipliers u+ of the working set
   creal zt[3], att[3];

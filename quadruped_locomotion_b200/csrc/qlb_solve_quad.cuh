@@ -124,6 +124,64 @@ __device__ __forceinline__ void solve6_thread(const real (&L)[21], const real (&
   }
 }
 
+// In-thread LDL' of a packed lower-triangular 6x6 SPD matrix; A <- L (strict lower part, unit diagonal), rd = 1/D.
+// The same pivots as chol6_thread (D_j is the square of its diagonal; a non-positive one is a failure), built row by
+// row from the unscaled row s_jk = L_jk D_k.  What differs is the dependent chain between two pivots: one reciprocal
+// (seed + two Newton steps, 4 dependent operations) and one FMA (D_j's last term s^2 / D_{j-1}) instead of a
+// reciprocal square root (6), the column scaling and an FMA.
+template <typename real>
+__device__ __forceinline__ bool ldl6_thread(real (&A)[21], real (&rd)[6]) {
+  bool ok = true;
+#pragma unroll
+  for (int j = 0; j < 6; j++) {
+    real s[6];
+#pragma unroll
+    for (int k = 0; k < 6; k++) {
+      if (k < j) {
+        real t = A[QLB_TRI(j, k)];
+#pragma unroll
+        for (int m = 0; m < 6; m++)
+          if (m < k) t = fma(-s[m], A[QLB_TRI(k, m)], t);
+        s[k] = t;
+      }
+    }
+    real d = A[QLB_TRI(j, j)];
+#pragma unroll
+    for (int k = 0; k < 6; k++) {
+      if (k < j) {
+        A[QLB_TRI(j, k)] = s[k] * rd[k];
+        d = (k + 1 < j) ? fma(-s[k], A[QLB_TRI(j, k)], d) : fma(-(s[k] * s[k]), rd[k], d);
+      }
+    }
+    ok = ok && (d > real(0.0));
+    rd[j] = fast_rcp(d);
+  }
+  return ok;
+}
+// L D L' x = b for the factors of ldl6_thread (x: b in, solution out).  Each substitution sums its terms with the one
+// that was computed last at the end of the chain.
+template <typename real>
+__device__ __forceinline__ void ldl6_solve(const real (&L)[21], const real (&rd)[6], real (&x)[6]) {
+#pragma unroll
+  for (int i = 1; i < 6; i++) {
+    real s = x[i];
+#pragma unroll
+    for (int k = 0; k < 6; k++)
+      if (k < i) s = fma(-L[QLB_TRI(i, k)], x[k], s);
+    x[i] = s;
+  }
+#pragma unroll
+  for (int i = 0; i < 6; i++) x[i] *= rd[i];
+#pragma unroll
+  for (int i = 4; i >= 0; i--) {
+    real s = x[i];
+#pragma unroll
+    for (int k = 5; k > 0; k--)
+      if (k > i) s = fma(-L[QLB_TRI(k, i)], x[k], s);
+    x[i] = s;
+  }
+}
+
 // One step of iterative refinement for (S^-1 + sum_legs sum_c al_c v_c v_c') t = rhs with the residual
 // evaluated through the factors v_c (not through the assembled matrix, whose large entries have already
 // rounded the S^-1 part away).  Used by the FP32 core only: it brings the solve from cond * eps ~ 5e-3
@@ -581,16 +639,31 @@ __device__ __forceinline__ void quad_output(const SolveArgsT<real>& a, const Leg
     if (a.netwrench) {
       // A x = sum over legs of A_k y_k (CFD.cpp:614-625)
       // (or, when the caller has the solution t of the 6x6 system: A x = b - S^-1 t, no reduction needed)
-      creal nwv[6];
+      // leg k writes components k and k+4 (k < 2)
+      creal nk, n4;
+      if (net_pre != nullptr) {
+        nk = solved ? sel4(leg, net_pre[0], net_pre[1], net_pre[2], net_pre[3]) : creal(0.0);
+        n4 = solved ? ((leg & 1) ? net_pre[5] : net_pre[4]) : creal(0.0);
+      } else {
+        // a reduce-scatter is enough: the lanes of even legs sum components 0, 2, 4 (exchanged across xor 1), those
+        // of odd legs 1, 3, 5, then a butterfly across xor 2 - (x0 + x1) + (x2 + x3), as quad_sum, with 6 values
+        // crossing lanes instead of 12
+        const bool odd = (leg & 1) != 0;
+        creal h[3];
 #pragma unroll
-      for (int r = 0; r < 6; r++) {
-        if (net_pre != nullptr) nwv[r] = solved ? net_pre[r] : creal(0.0);
-        else nwv[r] = quad_sum(live ? At[0][r] * y[0] + At[1][r] * y[1] + At[2][r] * y[2] : creal(0.0));
+        for (int i = 0; i < 3; i++) {
+          const creal ce = live ? At[0][2 * i] * y[0] + At[1][2 * i] * y[1] + At[2][2 * i] * y[2] : creal(0.0);
+          const creal co = live ? At[0][2 * i + 1] * y[0] + At[1][2 * i + 1] * y[1] + At[2][2 * i + 1] * y[2] : creal(0.0);
+          h[i] = (odd ? co : ce) + __shfl_xor_sync(kFull, odd ? ce : co, 1);
+        }
+#pragma unroll
+        for (int i = 0; i < 3; i++) h[i] += __shfl_xor_sync(kFull, h[i], 2);
+        nk = (leg & 2) ? h[1] : h[0];
+        n4 = h[2];
       }
       if (valid) {
-        // leg k writes components k and k+4 (k < 2)
-        a.netwrench[(size_t)leg * B + bq] = (real)sel4(leg, nwv[0], nwv[1], nwv[2], nwv[3]);
-        if (leg < 2) a.netwrench[(size_t)(4 + leg) * B + bq] = (real)((leg & 1) ? nwv[5] : nwv[4]);
+        a.netwrench[(size_t)leg * B + bq] = (real)nk;
+        if (leg < 2) a.netwrench[(size_t)(4 + leg) * B + bq] = (real)n4;
       }
     }
     {
