@@ -15,26 +15,29 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-Xcompiler", "-fPIC", "-shared", "--fmad=true", "-ldl"]
 
 
-def _stale() -> bool:
-    if not os.path.exists(LIB):
+def _stale(lib: str) -> bool:
+    if not os.path.exists(lib):
         return True
-    t = os.path.getmtime(LIB)
+    t = os.path.getmtime(lib)
     # every kernel header is included by qlb_api.cu: any edit under csrc/ or include/ makes the library stale
     deps = glob.glob(os.path.join(CSRC, "*.cu")) + glob.glob(os.path.join(CSRC, "*.cuh")) + \
         glob.glob(os.path.join(ROOT, "include", "*.h")) + [os.path.abspath(__file__)]
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, extra=()) -> str:
-    if not force and not _stale():
-        return LIB
+def build(force: bool = False, verbose: bool = False, extra=(), out: str | None = None) -> str:
+    """Compile libqlb.so.  extra: more nvcc flags (e.g. -DQLB_DBAS_MAX_ROUNDS=1 for a kernel variant); out: where the
+    library goes (default: in the package, where capi loads it from)."""
+    lib = LIB if out is None else os.path.abspath(out)
+    if not force and not _stale(lib):
+        return lib
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + list(extra) + ["-I" + os.path.join(ROOT, "include"), "-I" + CSRC, "-o", LIB] + \
+    cmd = [nvcc] + NVCC_FLAGS + list(extra) + ["-I" + os.path.join(ROOT, "include"), "-I" + CSRC, "-o", lib] + \
           [os.path.join(CSRC, s) for s in SOURCES]
     if verbose:
         print(" ".join(cmd))
     subprocess.check_call(cmd)
-    return LIB
+    return lib
 
 
 DEMO = os.path.join(PKG, "host", "tick_demo")

@@ -2,7 +2,6 @@
 """Build a kernel-variant copy of libqlb.so (experiments only): tools/build_variant.py NAME -DQLB_X=1 ...
 The library lands in quadruped_locomotion_b200/variants/libqlb_NAME.so; select it with QLB_LIB=<path>."""
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,10 +13,7 @@ def main():
     name, flags = sys.argv[1], sys.argv[2:]
     out = os.path.join(qb.PKG, "variants", f"libqlb_{name}.so")
     os.makedirs(os.path.dirname(out), exist_ok=True)
-    cmd = [os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")] + qb.NVCC_FLAGS + flags + \
-          ["-I" + os.path.join(ROOT, "include"), "-I" + qb.CSRC, "-o", out] + [os.path.join(qb.CSRC, s) for s in qb.SOURCES]
-    subprocess.check_call(cmd)
-    print(out)
+    print(qb.build(force=True, extra=flags, out=out))
 
 
 if __name__ == "__main__":
