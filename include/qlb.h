@@ -113,7 +113,11 @@ typedef enum qlb_state_status {
   QLB_STATE_OK = 0,            /* optimum found, KKT-verified active set */
   QLB_STATE_NO_STANCE = 1,     /* no leg in stance: nothing solved, outputs zero (CFD.cpp:127-132) */
   QLB_STATE_MAX_ITER = 2,      /* iteration limit hit; forces are the last iterate */
-  QLB_STATE_UNVERIFIED = 3,    /* converged, but the active-set polish failed its KKT check */
+  QLB_STATE_UNVERIFIED = 3,    /* converged, but the active-set polish failed its KKT check.  Both come only from the
+                                  interior point (the three-pass pipeline's second stage, the fused kernel's fallback),
+                                  whose start and stopping rule keep absolute scales: with forces far below 1 N or
+                                  weights far below the defaults it ends here more often (0.5 % of C3/C5 states at
+                                  (S, W) or (wrench, F_min) scaled by 2^-26 / 2^-30, three-pass pipeline) */
   QLB_STATE_BAD_INPUT = 4,     /* NaN/Inf input, degenerate surface normal, a joint angle beyond 1e6 rad, or a base
                                   quaternion / stance-leg surface normal that is not a unit vector (|v|^2 off by more than
                                   1e-5; smaller deviations - FP32 rounding - are renormalised); outputs zero */
@@ -162,7 +166,10 @@ int qlb_create(qlb_context** ctx, const qlb_leg_model legs[QLB_NUM_LEGS], const 
                int device, size_t max_batch);
 int qlb_destroy(qlb_context* ctx);
 /* Replaces ContactForceDistribution::loadParameters / VirtualModelController::loadParameters
- * (ContactForceDistribution.cpp:818-886, VirtualModelController.cpp:429-548). */
+ * (ContactForceDistribution.cpp:818-886, VirtualModelController.cpp:429-548).  Accepted (else
+ * QLB_ERR_INVALID_ARGUMENT, and the context keeps its parameters): W and every S_i in [1e-12, 1e12] with
+ * S_i / W <= 1e11, |F_min| <= 1e9, finite gravity, friction_default >= 0, ipm_tolerance > 0, ipm_max_iterations >= 1.
+ * The bound on S_i / W keeps the FP64 dual solve within ~1e-6 of the exact minimiser on every stance (qlb_api.cu). */
 int qlb_set_params(qlb_context* ctx, const qlb_params* params);
 int qlb_get_params(const qlb_context* ctx, qlb_params* params);
 

@@ -240,8 +240,16 @@ bool params_ok(const qlb_params* p) {
   const double lo = 1e-12, hi = 1e12;
   if (!(p->ground_force_weight >= lo && p->ground_force_weight <= hi) || !(p->ipm_tolerance > 0.0) || p->ipm_max_iterations < 1)
     return false;
-  for (int i = 0; i < 6; i++)
+  for (int i = 0; i < 6; i++) {
     if (!(p->wrench_weights[i] >= lo && p->wrench_weights[i] <= hi)) return false;  // the 6x6 dual system needs S^-1
+    // S_i / W <= 1e11.  The dual matrix S^-1 + A W^-1 A' has condition number ~S |A|^2 / W wherever the free columns of
+    // the wrench map do not span R^6 (one or two stance legs, legs pinned by active rows); the FP64 solve then loses
+    // ~2^-53 S |A|^2 / W of the forces (measured on B200 against a 50-digit reference: up to 5e-4 at W = 1e-12 with the
+    // default S), and at S / W = 1e16 its pivots drown in rounding (valid states reported QLB_STATE_BAD_INPUT at
+    // S = 1e12, W = 1e-4).  At the bound the loss is ~1e-6 (tests/test_solve_edges.py); the minimiser depends on S and
+    // W only through S / W.
+    if (!(p->wrench_weights[i] <= 1e11 * p->ground_force_weight)) return false;
+  }
   if (!(p->friction_default >= 0.0) || !std::isfinite(p->friction_default)) return false;
   if (!(std::fabs(p->min_normal_force) <= 1e9)) return false;
   return std::isfinite(p->gravity);

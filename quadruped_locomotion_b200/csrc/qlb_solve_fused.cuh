@@ -225,7 +225,6 @@ struct RoundState {
   creal y[3];       // primal iterate (y_n, y_1, y_2)
   creal u[3];       // multipliers of the rows held by the slots n, 1, 2 (0 where the slot is free)
   int a0, sg1, sg2; // working set: y_n pinned at F_min; y_1 = sg1 mu y_n; y_2 = sg2 mu y_n
-  float gscale;
   unsigned mask;
   bool alive;
   int rounds;
@@ -315,7 +314,8 @@ __device__ __forceinline__ void dbas_round(RoundState<creal>& q, const creal* b,
   up[2] = (alive && sg2 != 0) ? -sg2 * g2 : creal(0.0);
   up[0] = (alive && a0 != 0) ? g0 - mu * (up[1] + up[2]) : creal(0.0);
   // ---- ratio test: the step towards (y+, u+) that keeps every multiplier non-negative
-  const creal tol_u = Tol<creal>::mult() * (creal)q.gscale;
+  // (the scale of the gradient w y - A_k' t: the multipliers scale with W wherever the W term decides the internal forces)
+  const creal tol_u = Tol<creal>::mult() * quad_max_abs(att[0], att[1], att[2], cc.W * lane_max_abs(yp[0], yp[1], yp[2]));
   const bool act[3] = {alive && a0 != 0, alive && sg1 != 0, alive && sg2 != 0};
   creal tr[3], tl = creal(2.0);
 #pragma unroll
@@ -347,8 +347,7 @@ __device__ __forceinline__ void dbas_round(RoundState<creal>& q, const creal* b,
   creal e[5];
   leg_rows(yn3[0], yn3[1], yn3[2], mu, e);
   e[0] -= cc.fmin;
-  const float scale = fmaxf(1.f, quad_max(fmaxf(fabsf((float)yn3[0]), fmaxf(fabsf((float)yn3[1]), fabsf((float)yn3[2])))));
-  const creal tol_s = Tol<creal>::feas() * (creal)scale;
+  const creal tol_s = Tol<creal>::feas() * quad_max_abs(yn3[0], yn3[1], yn3[2]);
   bool viol = false;
   if (!blocked && alive) {
     if (na0 == 0 && e[0] < -tol_s) { na0 = 1; viol = true; }

@@ -40,6 +40,23 @@ __device__ __forceinline__ float quad_max(float v) {
   v = fmaxf(v, __shfl_xor_sync(kFull, v, 1));
   return fmaxf(v, __shfl_xor_sync(kFull, v, 2));
 }
+// max(|a|, |b|, |c|, |d|) over the quad, for the scales of tolerances.  A double is rounded down to its high word
+// (< 2^-20 relative): the high words of |x| order like the values, so the comparisons and the shuffles are 32-bit
+// integer work, off the FP64 pipe.  Scaling the inputs by a power of two scales the result exactly.
+__device__ __forceinline__ int abs_hi(const double x) { return __double2hiint(x) & 0x7fffffff; }
+__device__ __forceinline__ double from_hi(const int h) { return __hiloint2double(h, 0); }
+__device__ __forceinline__ float quad_max_abs(float a, float b, float c, float d = 0.f) {
+  return quad_max(fmaxf(fmaxf(fabsf(a), fabsf(b)), fmaxf(fabsf(c), fabsf(d))));
+}
+__device__ __forceinline__ double quad_max_abs(double a, double b, double c, double d = 0.0) {
+  int h = max(max(abs_hi(a), abs_hi(b)), max(abs_hi(c), abs_hi(d)));
+  h = max(h, __shfl_xor_sync(kFull, h, 1));
+  h = max(h, __shfl_xor_sync(kFull, h, 2));
+  return from_hi(h);
+}
+// max(|a|, |b|, |c|) of this lane (a double to its high word, as above)
+__device__ __forceinline__ float lane_max_abs(float a, float b, float c) { return fmaxf(fabsf(a), fmaxf(fabsf(b), fabsf(c))); }
+__device__ __forceinline__ double lane_max_abs(double a, double b, double c) { return from_hi(max(abs_hi(a), max(abs_hi(b), abs_hi(c)))); }
 __device__ __forceinline__ float quad_min(float v) {
   v = fminf(v, __shfl_xor_sync(kFull, v, 1));
   return fminf(v, __shfl_xor_sync(kFull, v, 2));
@@ -57,11 +74,13 @@ __device__ __forceinline__ unsigned quad_or(unsigned v) {
   return v | __shfl_xor_sync(kFull, v, 2);
 }
 
-// Tolerances of the two arithmetic types (relative to the force scale / the gradient scale of the state).
+// Tolerances of the two arithmetic types, relative to the scale of the quantity they judge, with no absolute floor
+// (a floor makes a state's result depend on the units of its inputs: forces of 1e-7 N against a 1 N floor of the
+// feasibility test, or multipliers that scale with W against a floor that does not).
 template <typename T> struct Tol;
 template <> struct Tol<double> {
-  __device__ static double feas() { return 1e-10; }   // a row counts as violated below -feas * scale
-  __device__ static double mult() { return 1e-13; }   // a multiplier counts as negative below -mult * gscale
+  __device__ static double feas() { return 1e-10; }   // a row counts as violated below -feas * max |y| of the state
+  __device__ static double mult() { return 1e-13; }   // a multiplier counts as negative below -mult * max(|W y|, |A' t|)
   __device__ static float ipm(float tol) { return tol; }
   static constexpr bool refine = false;
   static constexpr bool rescue = false;
@@ -230,7 +249,7 @@ struct LegSetup {
   real foot[3];    // foot position in base frame
   real b[6];       // desired wrench
   real mu, c0;     // friction coefficient; normal force of the strictly feasible interior-point start
-  float gscale, rm;  // scale of the linear term; 1 / number of constraint rows
+  float rm;          // 1 / number of constraint rows
   unsigned mask;
   int ns;
   bool alive, qbad, qinf;   // qinf: a stance leg has mu < 0 (no feasible force while F_min > 0)
@@ -459,10 +478,11 @@ __device__ __forceinline__ void quad_setup(const SolveArgsT<real>& a, const Devi
         E[0][c] = R[c] * nw[0] + R[3 + c] * nw[1] + R[6 + c] * nw[2];
         gb[c] = -prm.gravity * (real)R[6 + c];
       }
-      const creal ey[3] = {R[3], R[4], R[5]};
-      E[1][0] = E[0][1] * ey[2] - E[0][2] * ey[1];
-      E[1][1] = E[0][2] * ey[0] - E[0][0] * ey[2];
-      E[1][2] = E[0][0] * ey[1] - E[0][1] * ey[0];
+      // t1 = n x (R' e_y) = R' (n_w x e_y), and n_w x e_y = (-n_z, 0, n_x) is exact: rotated as one vector it keeps its
+      // direction to rounding however close the normal comes to the base y axis (the cross product of the two rotated
+      // vectors, each rounded on its own, loses the digits that cancel: 1e-10 of the frame at |n x e_y| = 1e-6)
+#pragma unroll
+      for (int c = 0; c < 3; c++) E[1][c] = R[6 + c] * nw[0] - R[c] * nw[2];
       creal rn = fast_rsqrt(E[1][0] * E[1][0] + E[1][1] * E[1][1] + E[1][2] * E[1][2]);
 #pragma unroll
       for (int c = 0; c < 3; c++) E[1][c] *= rn;
@@ -571,15 +591,6 @@ __device__ __forceinline__ void quad_setup(const SolveArgsT<real>& a, const Devi
     }
 #pragma unroll
     for (int c = 0; c < 3; c++) { L.nrm[c] = E[0][c]; L.foot[c] = footc[c]; }
-    float gsc = 0.f;
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-      creal g = creal(0.0);
-#pragma unroll
-      for (int r = 0; r < 6; r++) g = fma(At[c][r] * (creal)prm.S[r], L.b[r], g);
-      gsc = fmaxf(gsc, fabsf((float)g));
-    }
-    L.gscale = fmaxf(1.f, quad_max(gsc));
     L.c0 = fmax(fmax(creal(2.0) * (creal)prm.fmin, (L.b[0] * E[0][0] + L.b[1] * E[0][1] + L.b[2] * E[0][2]) * (ns > 0 ? creal(1.0) / ns : creal(0.0))),
                            (creal)prm.fmin + creal(1.0));
     L.rm = ns > 0 ? 1.f / (5.f * ns) : 0.f;
@@ -599,7 +610,7 @@ __device__ __forceinline__ void widen_setup(const LegSetup<real>& s, LegSetup<cr
 #pragma unroll
   for (int r = 0; r < 6; r++) d.b[r] = (creal)s.b[r];
   d.mu = (creal)s.mu; d.c0 = (creal)s.c0;
-  d.gscale = s.gscale; d.rm = s.rm; d.mask = s.mask; d.ns = s.ns; d.alive = s.alive; d.qbad = s.qbad; d.qinf = s.qinf;
+  d.rm = s.rm; d.mask = s.mask; d.ns = s.ns; d.alive = s.alive; d.qbad = s.qbad; d.qinf = s.qinf;
 }
 
 // value number `leg` of four, as two levels of selects (no divergent branches)
@@ -779,8 +790,7 @@ __device__ __forceinline__ void quad_first_solve(const LegSetup<creal>& L, const
   }
   leg_rows(y[0], y[1], y[2], L.mu, e);
   e[0] -= cfmin;
-  const float scale = fmaxf(1.f, quad_max(fmaxf(fabsf((float)y[0]), fmaxf(fabsf((float)y[1]), fabsf((float)y[2])))));
-  const creal tol_s = Tol<creal>::feas() * (creal)scale;
+  const creal tol_s = Tol<creal>::feas() * quad_max_abs(y[0], y[1], y[2]);
   bool viol = false;
 #pragma unroll
   for (int r = 0; r < 5; r++) viol = viol || (alive && e[r] < -tol_s);
@@ -910,7 +920,7 @@ __device__ __forceinline__ void quad_solve(const LegSetup<creal>& L, const CoreC
   const bool alive = L.alive;
   const int ns = L.ns;
   const creal mu = L.mu, c0 = L.c0;
-  const float gscale = L.gscale, rm = L.rm;
+  const float rm = L.rm;
   const bool qbad = L.qbad;
   const creal (&At)[3][6] = L.At;
   const creal (&b)[6] = L.b;
@@ -1101,8 +1111,8 @@ __device__ __forceinline__ void quad_solve(const LegSetup<creal>& L, const CoreC
       u[4] = (sg2 == 1) ? -g2 : creal(0.0);
       u[0] = (a0 != 0) ? g0 - mu * ((u[1] + u[2]) + (u[3] + u[4])) : creal(0.0);
       const bool act[5] = {a0 != 0, sg1 == -1, sg1 == 1, sg2 == -1, sg2 == 1};
-      const float scale = fmaxf(1.f, quad_max(fmaxf(fabsf((float)yp[0]), fmaxf(fabsf((float)yp[1]), fabsf((float)yp[2])))));
-      const creal tol_u = Tol<creal>::mult() * (creal)gscale, tol_s = Tol<creal>::feas() * (creal)scale;
+      const creal tol_s = Tol<creal>::feas() * quad_max_abs(yp[0], yp[1], yp[2]);
+      const creal tol_u = Tol<creal>::mult() * quad_max_abs(att[0], att[1], att[2], cc.W * lane_max_abs(yp[0], yp[1], yp[2]));
       // violations of this leg: negative multipliers (drop), else negative slacks (add; one per tangent pair)
       creal wd_v = -tol_u, wp_v = -tol_s;
       int wd_r = -1, wp_r = -1, nviol = 0;

@@ -99,7 +99,7 @@ struct WarpStash {
   creal* sl;      // [kStashLane][4 CAP]
   real* sj;       // [12][4 CAP]   Jacobian (9) and gravity torques (3); also the scratch of the tile phase
   creal* sb;      // [6][CAP]      desired wrench
-  uint32_t* sh;   // [4][CAP]      state index; mask | pattern << 4 | rounds << 24; gradient scale (float bits); spare
+  uint32_t* sh;   // [4][CAP]      state index; mask | pattern << 4 | rounds << 24; two spare words
   __device__ WarpStash(unsigned char* base) {
     using SL = StashLayout<real, creal, CAP>;
     sl = reinterpret_cast<creal*>(base);
@@ -116,7 +116,6 @@ __device__ __forceinline__ void stash_load(const WarpStash<real, creal, CAP>& ws
   const int e = 4 * slot + leg;
   const uint32_t w1 = ws.sh[CAP + slot];
   q.idx = ws.sh[slot];
-  q.gscale = __uint_as_float(ws.sh[2 * CAP + slot]);
   q.mask = w1 & 0xFu;
   q.alive = (w1 >> leg) & 1u;
   q.rounds = (int)(w1 >> 24);
@@ -185,7 +184,7 @@ __device__ __forceinline__ void round_phase(const SolveArgsT<real>& a, const Cor
     for (int r = 0; r < 6; r++) q.At[c][r] = creal(0.0);
     q.y[c] = creal(0.0); q.u[c] = creal(0.0);
   }
-  q.mu = creal(0.0); q.a0 = 0; q.sg1 = 0; q.sg2 = 0; q.gscale = 1.f; q.mask = 0u; q.alive = false; q.rounds = 0; q.idx = 0u;
+  q.mu = creal(0.0); q.a0 = 0; q.sg1 = 0; q.sg2 = 0; q.mask = 0u; q.alive = false; q.rounds = 0; q.idx = 0u;
   int slot = nth_set_bit(unassigned, quad);
   bool active = slot >= 0;
   {
@@ -391,7 +390,6 @@ qlb_single_kernel(const SolveArgsT<real> a, const __grid_constant__ FusedMaps ma
         if (leg == 0) {
           ws.sh[slot] = (unsigned)bq;
           ws.sh[CAP + slot] = L.mask | (pat << 4);
-          ws.sh[2 * CAP + slot] = __float_as_uint(L.gscale);
         }
       }
       occ |= __reduce_or_sync(kFull, hard ? (1u << slot) : 0u);

@@ -247,9 +247,11 @@ def test_nonpositive_minimal_force(solver, oracle, models, fmin):
 
 
 def test_parameter_bounds_are_enforced(solver):
-    """Weights outside [1e-12, 1e12], a negative default friction coefficient, NaN: qlb_set_params refuses them."""
+    """Weights outside [1e-12, 1e12], S_i / W above 1e11, a negative default friction coefficient, NaN: qlb_set_params
+    refuses them."""
     for field, val in (("ground_force_weight", 0.0), ("ground_force_weight", 1e13), ("friction_default", -0.1),
-                       ("min_normal_force", float("nan")), ("ground_force_weight", float("nan"))):
+                       ("min_normal_force", float("nan")), ("ground_force_weight", float("nan")),
+                       ("ground_force_weight", 1e-12), ("ground_force_weight", 9.9e-11)):
         p = solver.get_params()
         setattr(p, field, val)
         with pytest.raises(RuntimeError):
@@ -258,7 +260,16 @@ def test_parameter_bounds_are_enforced(solver):
     p.wrench_weights[2] = 1e-13
     with pytest.raises(RuntimeError):
         solver.set_params(p)
+    p = solver.get_params()
+    p.wrench_weights[3] = 1e12      # S_i / W = 1e16
+    with pytest.raises(RuntimeError):
+        solver.set_params(p)
     assert solver.get_params().ground_force_weight == 1e-4   # the context keeps its parameters
+    p = solver.get_params()
+    p.ground_force_weight = 1e-10   # max S_i / W = 1e11: the bound itself is accepted
+    solver.set_params(p)
+    p.ground_force_weight = 1e-4
+    solver.set_params(p)
 
 
 def test_huge_joint_angles_are_bad_input(solver):
